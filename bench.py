@@ -264,9 +264,10 @@ def launches_of(variant_fwd, variant_bwd, DH):
     }
 
 
-def measure_device(torch, dist, ops, _lib, name, K, W, dev, rank, world, reverse=False, on_device=False):
+def measure_device(torch, dist, ops, _lib, name, K, W, dev, rank, world, reverse=False, on_device=False, keep_outputs=False):
     """Device-resident arm of one workload: K steps between two CUDA events (CUDA-graph replay of one round over the rotating
-    input sets), then the same K steps eager with an event pair around every launch for the per-kernel durations."""
+    input sets), then the same K steps eager with an event pair around every launch for the per-kernel durations.
+    ``keep_outputs``: the result also carries "outputs", copies of what the last timed step computed."""
     B, NH, S, DH = WORKLOADS[name]
     alg = algorithmic(B, NH, S, DH)
     pk = peaks()
@@ -325,14 +326,16 @@ def measure_device(torch, dist, ops, _lib, name, K, W, dev, rank, world, reverse
             torch.cuda.synchronize()
 
     def run_steps(n, first):
+        """n steps; returns the plan of the last one."""
         if graph is not None:
             for _ in range(n // nsets):
                 graph.replay()
             for s_ in range(n - n % nsets, n):
                 step(plans[s_ % nsets])
-        else:
-            for s_ in range(n):
-                step(plans[(first + s_) % nsets])
+            return plans[(n - 1) % nsets]
+        for s_ in range(n):
+            step(plans[(first + s_) % nsets])
+        return plans[(first + n - 1) % nsets]
 
     if world > 1:
         dist.barrier()
@@ -340,12 +343,15 @@ def measure_device(torch, dist, ops, _lib, name, K, W, dev, rank, world, reverse
     t_start = torch.cuda.Event(enable_timing=True)
     t_end = torch.cuda.Event(enable_timing=True)
     t_start.record()
-    run_steps(K, W)
+    last = run_steps(K, W)
     t_end.record()
     torch.cuda.synchronize()
     if world > 1:
         dist.barrier()
     elapsed_ms = t_start.elapsed_time(t_end)
+    # copied before the passes below write the plans' output buffers again
+    outputs = {n_: t.clone() for n_, t in zip(("h", "dq", "dk", "dv", "di", "df"),
+                                              (last.h, last.dq, last.dk, last.dv, last.di, last.df))} if keep_outputs else None
     # The same K steps as eager launches through the plan's C-ABI calls (no graph): what the step costs with the host in the loop
     eager_value = None
     if graph is not None and world == 1:
@@ -399,8 +405,28 @@ def measure_device(torch, dist, ops, _lib, name, K, W, dev, rank, world, reverse
     return {
         "value": value, "ms_per_step": ms_per_step, "roofline": roofline, "launches_per_step": int(launches_per_step),
         "family": pl0.family, "nsets": nsets, "set_bytes": set_bytes, "graph": graph is not None, "plans": plans, "step": step,
-        "eager_value": eager_value,
+        "eager_value": eager_value, "outputs": outputs,
     }
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(torch, outputs, out_dir):
+    """Writes each output as ``out_dir/<name>.npy`` in float32 ((B, NH, S, DH) or (B, NH, S), the layout a caller of the cell
+    receives).  When they come to more than DUMP_BYTES together, each is replaced by a flat sample of its elements, the same
+    share of every output, at positions drawn from a fixed seed: two runs of the same workload sample the same elements."""
+    import numpy as np
+    total = sum(t.numel() for t in outputs.values()) * 4
+    budget = DUMP_BYTES - 256 * len(outputs)       # room for the .npy headers
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outputs.items():
+        t = t.float()
+        if total > budget:
+            n = t.numel() * budget // total
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:n].sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.contiguous().cpu().numpy())
 
 
 def measure_e2e(torch, dist, name, K, dev, rank, world, full_result):
@@ -500,19 +526,18 @@ def measure_e2e(torch, dist, name, K, dev, rank, world, full_result):
                 e2e_copy(s_ + 1)
             e2e_compute(s_)
 
-    Ke = max(3, min(K, 50))
     e2e_run(3)
     torch.cuda.synchronize()
     if world > 1:
         dist.barrier()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
-    e2e_run(Ke)
+    e2e_run(K)
     if back_stream is not main_stream:
         main_stream.wait_stream(back_stream)     # the result's way back to the host is inside the timed region
     e1.record()
     torch.cuda.synchronize()
-    e2e_ms = e0.elapsed_time(e1) / Ke
+    e2e_ms = e0.elapsed_time(e1) / K
     if world > 1:
         t = torch.tensor([e2e_ms], device=dev, dtype=torch.float64)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -532,6 +557,9 @@ def main():
     ap.add_argument("--cpu-sample-batch", type=int, default=8)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-also", action="store_true", help="skip the `also` block (the other BASELINE shapes)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step of the workload computed (h, dq, dk, dv, di, df) as DIR/<name>.npy, "
+                         "float32, at most 64 MB in all (a fixed sample of each output beyond that); the inputs are seeded")
     args = ap.parse_args()
     # stdout carries exactly one JSON line: whatever libraries print there (NCCL's version banner under NCCL_DEBUG=VERSION,
     # for one) is sent to stderr by pointing fd 1 at fd 2; emit() writes to the saved descriptor
@@ -564,7 +592,8 @@ def main():
     # ---- device-resident arm ("value") of the headline workload, clocks sampled during it --------
     sampler = ClockSampler(local_rank)
     sampler.start()
-    m = measure_device(torch, dist, ops, _lib, args.workload, K, W, dev, rank, world, reverse=bool(args.reverse))
+    m = measure_device(torch, dist, ops, _lib, args.workload, K, W, dev, rank, world, reverse=bool(args.reverse),
+                       keep_outputs=bool(args.dump_outputs) and rank == 0)
     # keep the sampler alive long enough for at least a few samples of a very short region
     t_hold = time.time()
     while len(sampler.samples) < 3 and time.time() - t_hold < 0.2:
@@ -573,6 +602,8 @@ def main():
     sampler.stop_flag = True
     sampler.join(timeout=1.0)
     del m["plans"]
+    if m["outputs"] is not None:
+        dump_outputs(torch, m.pop("outputs"), args.dump_outputs)
 
     # ---- end-to-end arm: the whole result comes back (headline); the checksum variant beside it --------
     e2e = measure_e2e(torch, dist, args.workload, K, dev, rank, world, full_result=True)
@@ -605,12 +636,11 @@ def main():
         also = []
         for name in ALSO_WORKLOADS:
             torch.cuda.empty_cache()
-            Ka = max(4, min(K, 12))
-            ma = measure_device(torch, dist, ops, _lib, name, Ka, 3, dev, rank, world, on_device=True)
+            ma = measure_device(torch, dist, ops, _lib, name, K, 3, dev, rank, world, on_device=True)
             del ma["plans"]
             Ba, NHa, Sa, DHa = WORKLOADS[name]
             also.append({"workload": name, "B_per_gpu": Ba, "NH": NHa, "S": Sa, "DH": DHa, "value": ma["value"], "unit": "tokens/s",
-                         "steps": Ka, "warmup": 3, "ms_per_step": ma["ms_per_step"], "gpu_launches": int(ma["launches_per_step"] * Ka),
+                         "steps": K, "warmup": 3, "ms_per_step": ma["ms_per_step"], "gpu_launches": int(ma["launches_per_step"] * K),
                          "roofline": ma["roofline"], "data": "synthetic, drawn on the device"})
         out["also"] = also
 

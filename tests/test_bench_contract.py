@@ -1,6 +1,7 @@
 """bench.py keeps the driver's JSON contract (one line on stdout, required keys) for both arms."""
 import json
 import os
+import re
 import subprocess
 import sys
 
@@ -59,7 +60,59 @@ def test_b200_arm_line():
     assert also["refdefault_B32_NH32_S1600_DH16"]["roofline"]["kernel"].startswith("tcgen05")   # zero-padded inside the library
     assert 0.7 < also["cfg3alt_B32_NH4_S1600_DH256"]["roofline"]["step_tensor_ceiling"] < 0.8
     for a in also.values():
+        assert a["steps"] == d["steps"]
         assert a["value"] > 0 and a["gpu_launches"] >= 2 * a["steps"] and 0 < a["roofline"]["step_hbm_frac"] < 1
     assert set(d["clocks"]) >= {"sm_mhz", "sm_max_mhz", "reasons"}
     cb = d["cpu_baseline"]
     assert cb["kind"] in ("reference", "port") and cb["value"] > 0 and "full batch" in cb["sample"]
+
+
+def test_dump_outputs_samples_the_same_elements_within_the_budget(tmp_path, monkeypatch):
+    import numpy as np
+    import torch
+    import bench
+    g = torch.Generator().manual_seed(0)
+    outs = {"h": torch.randn(2, 3, 50, 8, generator=g).bfloat16(), "di": torch.randn(2, 3, 50, generator=g)}
+    bench.dump_outputs(torch, outs, str(tmp_path / "whole"))
+    for name, t in outs.items():
+        got = np.load(tmp_path / "whole" / f"{name}.npy")
+        assert got.dtype == np.float32 and np.array_equal(got, t.float().numpy())
+    monkeypatch.setattr(bench, "DUMP_BYTES", 2000)
+    for tag in ("a", "b"):
+        bench.dump_outputs(torch, outs, str(tmp_path / tag))
+    files = [tmp_path / tag / f"{name}.npy" for tag in ("a", "b") for name in outs]
+    assert sum(os.path.getsize(f) for f in files[:2]) <= 2000
+    for name, t in outs.items():
+        a, b = (np.load(tmp_path / tag / f"{name}.npy") for tag in ("a", "b"))
+        assert a.ndim == 1 and 0 < a.size < t.numel() and np.array_equal(a, b)
+        assert np.isin(a, t.float().numpy().ravel()).all()
+
+
+@pytest.mark.gpu
+def test_b200_arm_dumps_the_last_steps_outputs(tmp_path):
+    import numpy as np
+    args = ("--steps", "3", "--warmup", "3", "--no-also", "--no-cpu-baseline")
+    for tag in ("a", "b"):
+        d = run(*args, "--dump-outputs", str(tmp_path / tag))
+    assert d["steps"] == 3
+    B, NH, S, DH = 32, 4, 400, 64
+    shapes = {"h": (B, NH, S, DH), "dq": (B, NH, S, DH), "dk": (B, NH, S, DH), "dv": (B, NH, S, DH), "di": (B, NH, S),
+              "df": (B, NH, S)}
+    assert sorted(os.listdir(tmp_path / "a")) == sorted(f"{n}.npy" for n in shapes)
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in os.listdir(tmp_path / "a")) <= 64e6
+    for name, shape in shapes.items():
+        a, b = (np.load(tmp_path / tag / f"{name}.npy") for tag in ("a", "b"))
+        assert a.dtype == np.float32 and a.shape == shape and np.isfinite(a).all() and np.abs(a).max() > 0
+        assert np.array_equal(a, b), name          # seeded inputs, deterministic kernels: the same arrays run to run
+    # the last timed step ran on input set (K - 1) mod nsets (graph replay) or (W + K - 1) mod nsets (eager launches)
+    import torch
+    import bench
+    from oracle import mlstm_oracle as O
+    nsets = int(re.search(r"rotate over (\d+) sets", d["config"]["l2"]).group(1))
+    last = (3 - 1 if d["config"]["launch"].startswith("CUDA graph") else d["warmup"] + 3 - 1) % nsets
+    ins = bench.make_inputs(torch, B, NH, S, DH, last, "cpu", torch.bfloat16)
+    want = O.mlstm_fwbw(*(t[:1].transpose(1, 2).double() for t in ins), chunk_size=64, eps=1e-6)
+    for name, w in zip(shapes, want):
+        got = torch.from_numpy(np.load(tmp_path / "a" / f"{name}.npy")[:1]).double()
+        err = float((got - w).abs().max() / w.abs().max())
+        assert err < (1e-2 if name == "h" else 2e-2), (name, err)
