@@ -321,9 +321,12 @@ int mlstm_b200_bwd_part(const mlstm_params* p, int part, void* cuda_stream);
 /* Name of the kernel family the call would dispatch to: "tcgen05" or "simt" (or NULL). */
 const char* mlstm_b200_kernel_name(const mlstm_params* p, int is_backward);
 
-/* Variant inside the family for this shape on the current device: "single_pass" (one CTA walks all
- * chunks of a (batch, head) pair, state on chip), "two_phase" / "chunk_parallel" (light sequential
- * state kernel + persistent chunk-parallel kernels, chunk states in `states`), or "simt". */
+/* Variant inside the family for this shape on the current device.  Forward: "single_pass" (one CTA
+ * walks all chunks of a (batch, head) pair, state on chip) or "two_phase" (light sequential state
+ * kernel + persistent chunk-parallel kernel, chunk states in `states`).  Backward: "fused_walk" (one
+ * CTA per (batch, head) pair walks the chunks in reverse from the chunk states in `states`) or
+ * "chunk_parallel" (persistent chunk-parallel kernels around one sequential adjoint-state kernel).
+ * "simt" for the SIMT family. */
 const char* mlstm_b200_kernel_variant(const mlstm_params* p, int is_backward);
 
 /* Kernels launched by this library in this process so far (for bench.py's gpu_launches). */

@@ -3,7 +3,6 @@ needs the -DMLSTM_TIMELINE build of mlstm_tc_bwd.cu:  python -c "from xlstm_yolo
 import os, sys
 import torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)))))
-os.environ["MLSTM_BWD_MERGE"] = "0"
 from xlstm_yolo_b200 import _lib
 _lib.LIB_PATH = _lib.LIB_PATH.replace("libmlstm_b200.so", "libmlstm_b200_tl.so")
 from xlstm_yolo_b200 import ops

@@ -1,6 +1,6 @@
 """Developer tool: forward + backward of the cell at head dims the tcgen05 kernels are not written for — DHqk = DHv / 2
 (mLSTMLayerVision's qk_dim_factor = 0.5), DH = 16 (the reference's default qkv_block_size), 32, 192: the zero-padded tensor-core
-path of mlstm_api.cu vs the fp32 SIMT family (MLSTM_NO_TCPAD=1)."""
+path of mlstm_api.cu."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)))))
 import torch

@@ -4,6 +4,7 @@ host-side mirrors of the reference interface (mLSTMBackend seam, MatrixLSTMCell)
 import copy
 import ctypes as C
 import inspect
+import itertools
 import os
 import pickle
 import re
@@ -145,6 +146,27 @@ def test_kernel_family_and_workspace(lib):
     assert lib.mlstm_b200_kernel_name(C.byref(p), 0) is None
     assert lib.mlstm_b200_kernel_variant(C.byref(p), 1) is None
     assert lib.mlstm_b200_kernel_variant(C.byref(_params()), 0) in (b"single_pass", b"two_phase")
+    # The dispatch table of the tensor-core family (the host library sees no device, so it sizes for 148 SMs): the forward
+    # is two-phase for head dim 256, and otherwise when 2 B NH <= 148 with >= 4 chunks; the backward is the fused walk iff
+    # the (padded) head dim is 64 or 128 and 2 B NH > 148.  The states buffer holds the chunk states unless a single-pass
+    # forward is called without saved rows; a padded head dim adds the padded initial / last states and, at DP = 256, the
+    # padded copies of q, k, v, h.
+    al = lambda x: (x + 255) & ~255
+    for (B, NH), S, DH in itertools.product([(1, 4), (8, 4), (37, 2), (32, 4), (75, 1)], [64, 384, 512, 1600],
+                                            [64, 128, 256, 16, 192]):
+        DP = 64 if DH <= 64 else (128 if DH <= 128 else 256)
+        two_phase = DP == 256 or (2 * B * NH <= 148 and S > 3 * 128)
+        fused = DP != 256 and 2 * B * NH > 148
+        items = B * NH * -(-S // 128)
+        for n_row in (None, 0x1000):
+            p = _params(B=B, NH=NH, S=S, DHQK=DH, DHV=DH)
+            p.n_row = p.m_row = n_row
+            assert lib.mlstm_b200_kernel_variant(C.byref(p), 0) == (b"two_phase" if two_phase else b"single_pass")
+            assert lib.mlstm_b200_kernel_variant(C.byref(p), 1) == (b"fused_walk" if fused else b"chunk_parallel")
+            states = al(items * (DP * DP * 2 + DP * 4 + 4)) if two_phase or n_row else 0
+            if DP != DH:
+                states += (4 * al(B * S * NH * DP * 2) if DP == 256 else 0) + 2 * al(B * NH * DP * DP * 4) + 2 * al(B * NH * DP * 4)
+            assert lib.mlstm_b200_state_bytes(C.byref(p)) == states, (B, NH, S, DH, n_row)
 
 
 def test_layer_tail_validation_needs_no_gpu(lib):

@@ -3,7 +3,6 @@
 #include <atomic>
 #include <cstdarg>
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 
 #include "mlstm_common.cuh"
@@ -33,7 +32,7 @@ void clear_error() { g_err[0] = 0; }
 // and the same leading block of the carried C, n.  The padded bf16 copies ((B, S, NH, DP), dense) of q, k, v and the padded h
 // live behind the chunk states in the caller's `states` buffer (written by the forward, read again by the backward); dh is
 // padded and dq, dk, dv are produced padded in the workspace and cropped out; initial / last states are padded / cropped the
-// same way; the 1 / sqrt(DHqk) scale is passed explicitly.  MLSTM_NO_TCPAD=1 keeps these shapes on the fp32 SIMT family.
+// same way; the 1 / sqrt(DHqk) scale is passed explicitly.
 // ---------------------------------------------------------------------------------------------------------------------
 namespace {
 
@@ -47,7 +46,7 @@ int padded_dim(const mlstm_params& p) {
 struct PadLayout {
   int DP;
   size_t inner, act, cst, nst;             // bytes: padded problem's own states | one padded activation | C | n
-  size_t act_s, act_w;                     // room per copy in the states buffer / in the workspace (0 where no copies are made)
+  size_t act_c;                            // room per copy in the states buffer and in the workspace (0 where none are made)
   size_t q_off, k_off, v_off, h_off, c0_off, n0_off, cl_off, nl_off, total;
   size_t ws_inner, dh_off, dq_off, dk_off, dv_off, ws_total;
 };
@@ -60,16 +59,10 @@ mlstm_params padded_params(const mlstm_params& p) {
 }
 
 // Where every access of a kernel variant to q, k, v, h, dh, dq, dk, dv goes through TMA, the padding costs nothing: the tensor
-// maps are encoded with the true row length and TMA supplies / clips the rest (tc_tmap.cuh: ExtentOverride).  That holds for the
-// DP = 64 and 128 kernels except the two-walk single-pass backward (mlstm_tc_bwd1p.cu): where they touch rows with plain loads
-// or stores (the two-phase forward's h rows, tc_dn_kernel, two row reads of the DH = 128 fused walk) they take the true row
-// length as an argument; the DH = 256 family and the single-pass backward run on the copies.  MLSTM_TCPAD_COPY=1 forces the copies.
-bool zero_copy_off() {
-  static const bool off = getenv("MLSTM_TCPAD_COPY") != nullptr && getenv("MLSTM_TCPAD_COPY")[0] == '1';
-  return off;
-}
-bool zero_copy_fwd(const mlstm_params& pp) { return !zero_copy_off() && pp.DHV <= 128; }
-bool zero_copy_bwd(const mlstm_params& pp) { return !zero_copy_off() && pp.DHV <= 128 && !tc_use_single_pass_bwd(pp); }
+// maps are encoded with the true row length and TMA supplies / clips the rest (tc_tmap.cuh: ExtentOverride).  That holds for
+// every DP = 64 and 128 kernel: where they touch rows with plain loads or stores (the two-phase forward's h rows, tc_dn_kernel,
+// two row reads of the DH = 128 fused walk) they take the true row length as an argument.  The DH = 256 family runs on copies.
+bool zero_copy(const mlstm_params& pp) { return pp.DHV <= 128; }
 
 PadLayout pad_layout(const mlstm_params& p) {
   const mlstm_params pp = padded_params(p);
@@ -79,31 +72,28 @@ PadLayout pad_layout(const mlstm_params& p) {
   l.act = al256((size_t)p.B * p.S * p.NH * l.DP * 2);
   l.cst = al256((size_t)p.B * p.NH * l.DP * l.DP * 4);
   l.nst = al256((size_t)p.B * p.NH * l.DP * 4);
-  // copies of q, k, v, h: made by a forward that needs them, or by the backward that follows a copy-free forward (n_row set =
-  // a backward will follow; the backward itself always sees n_row, so both calls lay the buffer out the same way)
-  l.act_s = (!zero_copy_fwd(pp) || (p.n_row != nullptr && !zero_copy_bwd(pp))) ? l.act : 0;
-  l.act_w = !zero_copy_bwd(pp) ? l.act : 0;
+  // copies of q, k, v, h (made by the forward, read again by the backward) and of dh, dq, dk, dv
+  l.act_c = zero_copy(pp) ? 0 : l.act;
   l.q_off = l.inner;
-  l.k_off = l.q_off + l.act_s;
-  l.v_off = l.k_off + l.act_s;
-  l.h_off = l.v_off + l.act_s;
-  l.c0_off = l.h_off + l.act_s;
+  l.k_off = l.q_off + l.act_c;
+  l.v_off = l.k_off + l.act_c;
+  l.h_off = l.v_off + l.act_c;
+  l.c0_off = l.h_off + l.act_c;
   l.n0_off = l.c0_off + l.cst;
   l.cl_off = l.n0_off + l.nst;
   l.nl_off = l.cl_off + l.cst;
   l.total = l.nl_off + l.nst;
   l.ws_inner = al256(tc_bwd_workspace(pp));
   l.dh_off = l.ws_inner;
-  l.dq_off = l.dh_off + l.act_w;
-  l.dk_off = l.dq_off + l.act_w;
-  l.dv_off = l.dk_off + l.act_w;
-  l.ws_total = l.dv_off + l.act_w;
+  l.dq_off = l.dh_off + l.act_c;
+  l.dk_off = l.dq_off + l.act_c;
+  l.dv_off = l.dk_off + l.act_c;
+  l.ws_total = l.dv_off + l.act_c;
   return l;
 }
 
 bool pad_path(const mlstm_params& p) {
-  static const bool off = getenv("MLSTM_NO_TCPAD") != nullptr && getenv("MLSTM_NO_TCPAD")[0] == '1';
-  if (off || p.dtype != MLSTM_BF16 || p.DHQK % 8 != 0 || p.DHV % 8 != 0 || p.DHQK < 16 || p.DHV < 16) return false;
+  if (p.dtype != MLSTM_BF16 || p.DHQK % 8 != 0 || p.DHV % 8 != 0 || p.DHQK < 16 || p.DHV < 16) return false;
   if (padded_dim(p) == 0 || tc_supported(p)) return false;
   return tc_supported(padded_params(p));
 }
@@ -211,8 +201,8 @@ int make_padded(const mlstm_params& p, int is_bwd, mlstm_params* out, PadLayout*
   pp.states_bytes = l.inner;
   if (l.inner == 0) pp.states = nullptr;   // forward-only single-pass call: the padded problem keeps its states on chip
   // a side that already has the padded width runs on the caller's own tensors (DHqk < DHv = DP: only q, k are copied);
-  // so does everything in the zero-copy variants
-  const bool zc = is_bwd ? zero_copy_bwd(pp) : zero_copy_fwd(pp);
+  // so does everything at DP = 64 and 128
+  const bool zc = zero_copy(pp);
   const bool pad_qk = p.DHQK != l.DP && !zc, pad_v = p.DHV != l.DP && !zc;
   if (pad_qk) { pp.q = dense_act(sb + l.q_off, p, l.DP); pp.k = dense_act(sb + l.k_off, p, l.DP); }
   if (pad_v) { pp.v = dense_act(sb + l.v_off, p, l.DP); pp.h = dense_act(sb + l.h_off, p, l.DP); }
@@ -234,7 +224,7 @@ int tcpad_fwd(const mlstm_params& p, cudaStream_t st) {
   PadLayout l;
   int rc = make_padded(p, 0, &pp, &l);
   if (rc) return rc;
-  const bool zc = zero_copy_fwd(pp);
+  const bool zc = zero_copy(pp);
   const bool pad_qk = p.DHQK != l.DP && !zc, pad_v = p.DHV != l.DP && !zc;
   ExtentScope ext;
   if (zc) {
@@ -267,20 +257,13 @@ int tcpad_bwd(const mlstm_params& p, cudaStream_t st, int part) {
   PadLayout l;
   int rc = make_padded(p, 1, &pp, &l);   // q, k, v, h, the initial states: the copies the forward left in the states buffer
   if (rc) return rc;
-  const bool zc = zero_copy_bwd(pp);
+  const bool zc = zero_copy(pp);
   const bool pad_qk = p.DHQK != l.DP && !zc, pad_v = p.DHV != l.DP && !zc;
   ExtentScope ext;
   if (zc) {
     ext.add(p.q.ptr, p.DHQK); ext.add(p.k.ptr, p.DHQK); ext.add(p.dq.ptr, p.DHQK); ext.add(p.dk.ptr, p.DHQK);
     ext.add(p.v.ptr, p.DHV); ext.add(p.h.ptr, p.DHV); ext.add(p.dh.ptr, p.DHV); ext.add(p.dv.ptr, p.DHV);
     return tc_bwd(pp, st, part);
-  }
-  if (zero_copy_fwd(pp)) {   // the forward ran on the caller's tensors and left no copies behind: make them now
-    if ((pad_qk || pad_v) &&
-        (rc = pad_rows(p, l.DP, pad_qk ? job(p.q, pp.q, p.DHQK) : no_job(), pad_qk ? job(p.k, pp.k, p.DHQK) : no_job(),
-                       pad_v ? job(p.v, pp.v, p.DHV) : no_job(), 1, st, "pad_rows")))
-      return rc;
-    if (pad_v && (rc = pad_rows(p, l.DP, job(p.h, pp.h, p.DHV), no_job(), no_job(), 1, st, "pad_rows"))) return rc;
   }
   if (pad_v && (rc = pad_rows(p, l.DP, job(p.dh, pp.dh, p.DHV), no_job(), no_job(), 1, st, "pad_rows"))) return rc;
   if ((rc = tc_bwd(pp, st, part))) return rc;
@@ -452,7 +435,7 @@ const char* mlstm_b200_kernel_variant(const mlstm_params* p, int is_backward) {
   if (pick(*p) == FAM_TCPAD) { pp_ = padded_params(*p); p = &pp_; }
   switch (pick(*p)) {
     case FAM_TC:
-      if (is_backward) return tc_use_fused_bwd(*p) ? "fused_walk" : (tc_use_single_pass_bwd(*p) ? "single_pass" : "chunk_parallel");
+      if (is_backward) return tc_use_fused_bwd(*p) ? "fused_walk" : "chunk_parallel";
       return tc_use_two_phase(*p) ? "two_phase" : "single_pass";
     case FAM_SIMT: return "simt";
     default: return nullptr;

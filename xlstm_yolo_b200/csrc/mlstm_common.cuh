@@ -25,7 +25,6 @@ int tc_bwd(const mlstm_params& p, cudaStream_t st, int part = -1);
 size_t tc_bwd_workspace(const mlstm_params& p);
 size_t tc_state_bytes(const mlstm_params& p);
 bool tc_use_two_phase(const mlstm_params& p);
-bool tc_use_single_pass_bwd(const mlstm_params& p);
 bool tc_use_fused_bwd(const mlstm_params& p);
 bool tc_supported(const mlstm_params& p);
 
@@ -58,11 +57,6 @@ __device__ __forceinline__ float igate_dlog(const mlstm_params& p, float i_raw) 
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-  return v;
-}
-__device__ __forceinline__ float warp_max(float v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
   return v;
 }
 // Fixed-order (deterministic) sum of n_part partials spaced `stride` floats apart, by a group of 8 adjacent lanes: lane l adds

@@ -11,8 +11,6 @@
 //     N = 32 / 48 MMA per k-step accumulates all three, the epilogue adds them — fp32 weights at fp32 accuracy, as the SIMT kernel;
 //   * two TMEM accumulators alternate between tiles, so the epilogue of one tile (128 threads: one token row each, bias, two
 //     float4 stores) runs under the MMAs of the next.
-#include <cstdlib>
-
 #include "tc_common.cuh"
 
 namespace mlstm {
@@ -160,8 +158,7 @@ __global__ void __launch_bounds__(GT_NT, 1) gates_fwd_tc_kernel(const __grid_con
 }  // namespace
 
 bool gates_tc_ok(const mlstm_gate_proj_params& p) {
-  static const bool off = getenv("MLSTM_GATES_TC") != nullptr && getenv("MLSTM_GATES_TC")[0] == '0';
-  if (off || p.dtype != MLSTM_BF16 || p.D % 64 != 0 || 2 * p.NH > 16 || p.ld % 8 != 0) return false;
+  if (p.dtype != MLSTM_BF16 || p.D % 64 != 0 || 2 * p.NH > 16 || p.ld % 8 != 0) return false;
   // TMA needs 16-byte aligned base addresses; views that start mid-row at an odd offset stay on the SIMT kernel
   if (((reinterpret_cast<uintptr_t>(p.q) | reinterpret_cast<uintptr_t>(p.k) | reinterpret_cast<uintptr_t>(p.v)) & 15u) != 0) return false;
   const size_t wbytes = (size_t)(3 * p.D / 64) * (2 * p.NH > 8 ? 48 : 32) * 128;

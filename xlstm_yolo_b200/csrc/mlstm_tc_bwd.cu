@@ -17,8 +17,6 @@
 // CPU emulation in tests/emu_kernel_dataflow.py.)  The parallel kernels share one skeleton:
 // MMA1 (128x128 tile product) -> SIMT gating into a bf16 tile -> MMA2, with 16 compute warps,
 // one control warp issuing all TMA / tcgen05.mma, one gate warp preparing the next item.
-#include <cstdlib>
-
 #include "tc_common.cuh"
 
 namespace mlstm {
@@ -120,7 +118,7 @@ struct SmemB {
 // in one launch, each on its own slice of the grid — see tc_bwd_b12_kernel)
 template <int DH, int MODE>
 __device__ __forceinline__ void par_body(const BwdMaps& maps, const mlstm_params& p, const float scale, const int n_items,
-                                         const int order, const int cta, const int ncta, const bool write_dn = true) {
+                                         const int cta, const int ncta, const bool write_dn = true) {
   constexpr int KT = DH / 64;
   constexpr int TILE_C = SmemB<DH>::TILE_C;
   constexpr int NB = DH / 32;
@@ -208,15 +206,9 @@ __device__ __forceinline__ void par_body(const BwdMaps& maps, const mlstm_params
     __syncwarp();
   };
 
-  // Work order.  Items are (batch*head, chunk) pairs with linear id bh*NC + sc.  order 0 walks them
-  // head-major; 1 / 2 walk them chunk-major, ascending / descending chunk index.
-  const int n_bh = p.B * p.NH;
-  auto lin_of = [&](int i) {
-    if (order == 0 || i >= n_items) return i;
-    const int c = i / n_bh, bh_ = i - c * n_bh;
-    return bh_ * NC + (order == 1 ? c : NC - 1 - c);
-  };
-  const int item0 = lin_of(cta);   // ncta is never larger than n_items
+  // Items are (batch*head, chunk) pairs with id bh*NC + sc, walked head-major: this CTA takes cta, cta + ncta, ...
+  // (measured on B200: no chunk-major order beats it; the kernels are not DRAM-bound)
+  const int item0 = cta;   // ncta is never larger than n_items
   if (issuer) {
     load_act(sm.t0, &maps.t0, &sm.bar_t0, item0); load_act(sm.t1, &maps.t1, &sm.bar_t1, item0);
     load_st(item0); load_act(sm.t2, &maps.t2, &sm.bar_t2, item0);
@@ -225,7 +217,7 @@ __device__ __forceinline__ void par_body(const BwdMaps& maps, const mlstm_params
   }
   if (gatew) {
     prep_item(item0, 0);
-    if (cta + ncta < n_items) prep_item(lin_of(cta + ncta), 1);
+    if (cta + ncta < n_items) prep_item(cta + ncta, 1);
   }
   __syncthreads();
   if (issuer) {
@@ -241,15 +233,14 @@ __device__ __forceinline__ void par_body(const BwdMaps& maps, const mlstm_params
   long long* tlb = reinterpret_cast<long long*>(MLSTM_TL_MODE == 0 ? ws_kpart : ws_rpart);
 #endif
   int n = 0;
-  for (int it = cta; it < n_items; it += ncta, ++n) {
-    const int item = lin_of(it);
+  for (int item = cta; item < n_items; item += ncta, ++n) {
     TLB(0);
     const uint32_t ph = n & 1;
     const uint32_t tS = IS_A ? tm + ph * 128 : tm;   // B: S is dead once the gated tile is built, one buffer suffices
-    const bool has_next = it + ncta < n_items;
-    const int next = lin_of(it + ncta);
+    const int next = item + ncta;
+    const bool has_next = next < n_items;
     if (gatew) {
-      if (it + 2 * ncta < n_items) prep_item(lin_of(it + 2 * ncta), (n + 2) % 3);
+      if (item + 2 * ncta < n_items) prep_item(item + 2 * ncta, (n + 2) % 3);
       __syncthreads();
       continue;
     }
@@ -465,8 +456,8 @@ __device__ __forceinline__ void par_body(const BwdMaps& maps, const mlstm_params
 
 template <int DH, int MODE>
 __global__ void __launch_bounds__(NT, 1) tc_bwd_par_kernel(const __grid_constant__ BwdMaps maps, const mlstm_params p,
-                                                           const float scale, const int n_items, const int order) {
-  par_body<DH, MODE>(maps, p, scale, n_items, order, blockIdx.x, gridDim.x);
+                                                           const float scale, const int n_items) {
+  par_body<DH, MODE>(maps, p, scale, n_items, blockIdx.x, gridDim.x);
 }
 
 // B1 (dv) and B2 (dk) side by side in one launch: CTAs [0, n_b2) run B2, the rest run B1, both walking
@@ -476,9 +467,9 @@ __global__ void __launch_bounds__(NT, 1) tc_bwd_par_kernel(const __grid_constant
 template <int DH>
 __global__ void __launch_bounds__(NT, 1) tc_bwd_b12_kernel(const __grid_constant__ BwdMaps maps1, const __grid_constant__ BwdMaps maps2,
                                                            const mlstm_params p, const float scale, const int n_items,
-                                                           const int order, const int n_b2) {
-  if ((int)blockIdx.x < n_b2) par_body<DH, MODE_B2>(maps2, p, scale, n_items, order, blockIdx.x, n_b2);
-  else par_body<DH, MODE_B1>(maps1, p, scale, n_items, order, blockIdx.x - n_b2, gridDim.x - n_b2);
+                                                           const int n_b2) {
+  if ((int)blockIdx.x < n_b2) par_body<DH, MODE_B2>(maps2, p, scale, n_items, blockIdx.x, n_b2);
+  else par_body<DH, MODE_B1>(maps1, p, scale, n_items, blockIdx.x - n_b2, gridDim.x - n_b2);
 }
 
 // =============================================================================================
@@ -757,9 +748,9 @@ __global__ void __launch_bounds__(NT, 1) tc_state_bwd_kernel(const __grid_consta
 template <int DH>
 __global__ void __launch_bounds__(NT, 1) tc_bwd_sa_kernel(const __grid_constant__ BwdMaps maps_s, const __grid_constant__ BwdMaps maps_a,
                                                           const mlstm_params p, const float scale, const int n_items,
-                                                          const int order, const int n_state) {
+                                                          const int n_state) {
   if ((int)blockIdx.x < n_state) state_bwd_body<DH>(maps_s, p, scale, blockIdx.x, 0);
-  else par_body<DH, MODE_A>(maps_a, p, scale, n_items, order, blockIdx.x - n_state, gridDim.x - n_state, false);
+  else par_body<DH, MODE_A>(maps_a, p, scale, n_items, blockIdx.x - n_state, gridDim.x - n_state, false);
 }
 
 // dn_t = dnf_t (dh_t . h_t) for every row (the same formula as kernel A and gates_warp_bwd): DH / 8 lanes per row, one 16-byte
@@ -875,14 +866,6 @@ int launched(const char* name) {
   return MLSTM_OK;
 }
 
-// item order of kernels A, B1, B2 (see lin_of); MLSTM_BWD_ORDER="abc" (digits 0-2) overrides for experiments
-int order_of(int k) {
-  static const char* env = getenv("MLSTM_BWD_ORDER");
-  static const int dflt[3] = {0, 0, 0};   // measured on B200: no order beats head-major (the kernels are not DRAM-bound)
-  if (env && env[0] && env[1] && env[2] && env[k] >= '0' && env[k] <= '2') return env[k] - '0';
-  return dflt[k];
-}
-
 template <int DH>
 int launch_bwd(const mlstm_params& p, cudaStream_t st, int part) {
   const StateLayout slay(p.B, p.NH, p.S, DH);
@@ -914,9 +897,8 @@ int launch_bwd(const mlstm_params& p, cudaStream_t st, int part) {
   const size_t smB = sizeof(SmemB<DH>), smSB = sizeof(SmemSB<DH>);
   int rc;
   // whole backward in one call with few (batch, head) pairs: the state walk and kernel A share a launch (tc_bwd_sa_kernel)
-  static const bool merge_off = getenv("MLSTM_BWD_MERGE") != nullptr && getenv("MLSTM_BWD_MERGE")[0] == '0';
   const int n_state = p.B * p.NH;
-  const bool merged = part != 0 && part != 1 && !merge_off && 2 * n_state <= sms && NC > 1 && (int64_t)n_state * p.S < (1ll << 31);
+  const bool merged = part != 0 && part != 1 && 2 * n_state <= sms && NC > 1 && (int64_t)n_state * p.S < (1ll << 31);
   if (merged) {
     const int64_t rows = (int64_t)n_state * p.S;
     const int rows_per_cta = 8 * (32 / (DH / 8)) * DN_U;
@@ -928,13 +910,13 @@ int launch_bwd(const mlstm_params& p, cudaStream_t st, int part) {
     const size_t smSA = smB > smSB ? smB : smSB;
     const int n_a = n_items < sms - n_state ? n_items : sms - n_state;
     if ((rc = prep(tc_bwd_sa_kernel<DH>, smSA, "tc_bwd_state_dq"))) return rc;
-    tc_bwd_sa_kernel<DH><<<dim3(n_state + n_a), dim3(NT), smSA, st>>>(ms, ma, p, scale, n_items, order_of(0), n_state);
+    tc_bwd_sa_kernel<DH><<<dim3(n_state + n_a), dim3(NT), smSA, st>>>(ms, ma, p, scale, n_items, n_state);
     if ((rc = launched("tc_bwd_state_dq"))) return rc;
   }
   if (part != 1 && !merged) {
     BwdMaps m{mdh, mv, mk, mcs, mq, mh, mdq};
     if ((rc = prep(tc_bwd_par_kernel<DH, MODE_A>, smB, "tc_bwd_dq"))) return rc;
-    tc_bwd_par_kernel<DH, MODE_A><<<dim3(grid), dim3(NT), smB, st>>>(m, p, scale, n_items, order_of(0));
+    tc_bwd_par_kernel<DH, MODE_A><<<dim3(grid), dim3(NT), smB, st>>>(m, p, scale, n_items);
     if ((rc = launched("tc_bwd_dq"))) return rc;
   }
   if (part != 0) {
@@ -949,16 +931,16 @@ int launch_bwd(const mlstm_params& p, cudaStream_t st, int part) {
     if (n_items < 4 * sms) {
       // few items per CTA: two full-width launches balance better than two half-width groups
       if ((rc = prep(tc_bwd_par_kernel<DH, MODE_B1>, smB, "tc_bwd_dv"))) return rc;
-      tc_bwd_par_kernel<DH, MODE_B1><<<dim3(grid), dim3(NT), smB, st>>>(m1, p, scale, n_items, order_of(1));
+      tc_bwd_par_kernel<DH, MODE_B1><<<dim3(grid), dim3(NT), smB, st>>>(m1, p, scale, n_items);
       if ((rc = launched("tc_bwd_dv"))) return rc;
       if ((rc = prep(tc_bwd_par_kernel<DH, MODE_B2>, smB, "tc_bwd_dk"))) return rc;
-      tc_bwd_par_kernel<DH, MODE_B2><<<dim3(grid), dim3(NT), smB, st>>>(m2, p, scale, n_items, order_of(2));
+      tc_bwd_par_kernel<DH, MODE_B2><<<dim3(grid), dim3(NT), smB, st>>>(m2, p, scale, n_items);
       if ((rc = launched("tc_bwd_dk"))) return rc;
     } else {
       // B2 costs ~1.2x B1 per item: it gets the larger share of the CTAs
       const int n_b2 = (sms * 6 + 5) / 11;
       if ((rc = prep(tc_bwd_b12_kernel<DH>, smB, "tc_bwd_dkdv"))) return rc;
-      tc_bwd_b12_kernel<DH><<<dim3(sms), dim3(NT), smB, st>>>(m1, m2, p, scale, n_items, order_of(1), n_b2);
+      tc_bwd_b12_kernel<DH><<<dim3(sms), dim3(NT), smB, st>>>(m1, m2, p, scale, n_items, n_b2);
       if ((rc = launched("tc_bwd_dkdv"))) return rc;
     }
     tc_dfscan_kernel<<<dim3(n_items), dim3(L), 0, st>>>(p, DH);
@@ -992,13 +974,6 @@ void tc_bwd_layout(const mlstm_params& p, size_t* dn_off, size_t* rpart_off, siz
   *total = b.total;
 }
 
-// Short sequences with enough (batch, head) pairs to fill the GPU keep the single-pass kernels
-// (mlstm_tc_bwd1p.cu): with <= 4 chunks per head the serial chain is short and the chunk-state
-// round trip through HBM does not pay.
-size_t tc_bwd1p_workspace(const mlstm_params& p);
-int tc_bwd1p(const mlstm_params& p, cudaStream_t st, int part);
-bool tc_use_single_pass_bwd(const mlstm_params& p);
-
 size_t tc_bwd_fused_workspace(const mlstm_params& p);
 int tc_bwd_fused(const mlstm_params& p, cudaStream_t st, int part);
 size_t tc_bwd_fused128_workspace(const mlstm_params& p);
@@ -1006,7 +981,7 @@ int tc_bwd_fused128(const mlstm_params& p, cudaStream_t st, int part);
 
 size_t tc_bwd_workspace(const mlstm_params& p) {
   if (tc_use_fused_bwd(p)) return p.DHQK == 64 ? tc_bwd_fused_workspace(p) : tc_bwd_fused128_workspace(p);
-  return tc_use_single_pass_bwd(p) ? tc_bwd1p_workspace(p) : BwdLayout(p.B, p.NH, p.S, p.DHQK).total;
+  return BwdLayout(p.B, p.NH, p.S, p.DHQK).total;
 }
 
 int tc256_bwd(const mlstm_params& p, cudaStream_t st, int part);
@@ -1014,7 +989,6 @@ int tc256_bwd(const mlstm_params& p, cudaStream_t st, int part);
 int tc_bwd(const mlstm_params& p, cudaStream_t st, int part) {
   if (p.DHQK == 256) return tc256_bwd(p, st, part);
   if (tc_use_fused_bwd(p)) return p.DHQK == 64 ? tc_bwd_fused(p, st, part) : tc_bwd_fused128(p, st, part);
-  if (tc_use_single_pass_bwd(p)) return tc_bwd1p(p, st, part);
   if (p.DHQK == 64) return launch_bwd<64>(p, st, part);
   return launch_bwd<128>(p, st, part);
 }

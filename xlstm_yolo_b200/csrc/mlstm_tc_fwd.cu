@@ -1,11 +1,10 @@
 // tcgen05 / TMEM / TMA forward kernel of the mLSTM cell for bf16 I/O, DH in {64, 128}.
 //
 // One CTA per (batch, head) walks the sequence in chunks of L = 128 tokens with the (C, n, m)
-// state resident on chip.  21 warps in three roles:
-//   16 compute warps  warp w owns tile rows / TMEM lanes 32*(w%4)..+31 and the 32-column block
-//                     w/4 of every 128-wide matrix (one 32x32 block of S, H, G, C per warp)
-//    1 control warp   lane 0 issues every TMA load/store and every tcgen05.mma (pre-built
-//                     descriptors), so no compute warp ever sits in an issue loop
+// state resident on chip.  18 warps in three roles:
+//   16 compute warps  two groups of 8 (below); warp w owns tile rows / TMEM lanes 32*(w%4)..+31
+//    1 control warp   lane 0 issues every TMA load/store and the S, H and C MMAs (pre-built descriptors),
+//                     so no compute warp ever sits in an issue loop
 //    1 gate warp      log-sigmoid cumsum / running-max scans of the gates, two chunks ahead
 //   C  : fp32 accumulator in TMEM, updated by an accumulating MMA  C += Kbar^T V
 //   Cb : bf16 copy of C in shared memory (MN-major B operand of  G = Q Cb)
@@ -21,8 +20,14 @@
 //   SIMT  Cb <- bf16(C),  C <- decay_next * C   (one TMEM pass per chunk)
 // No intermediate (D matrix, gates, P) ever reaches HBM.  `reverse` walks the tokens from
 // the end: tiles stay in memory order, the causal mask and the gate scans flip.
-#include <cstdlib>
-
+//
+// The two compute groups work on the two dependency chains of a chunk concurrently:
+//   group A (warps 0-7)   the score chain    wait S -> P = S * exp2(u - M) -> [MMA2 H = P V] -> h = (H + w G) / N
+//   group B (warps 8-15)  the state chain    q . n_prev -> Kbar = kw K -> [state MMA] -> Cb <- bf16(C), C <- decay C, n
+// A warp owns one half of the columns (two 32-column blocks).  The control lane polls the two hand-offs (P written, Kbar
+// written) and issues MMA2 / the state MMA in whichever order they become ready; n += Kbar^T 1 goes out from a lane of
+// group B, G = Q Cb from lane 0 of warp 1 once the state pass has refreshed Cb.  One CTA-wide barrier per chunk remains
+// (gate ring, G of the next chunk after the state pass).  h is staged in its own tile (the state chain may still read K).
 #include "tc_common.cuh"   // StateLayout / store_row32 (the per-chunk state buffer shared with the backward)
 
 namespace mlstm {
@@ -39,18 +44,6 @@ constexpr float LOG2E = 1.4426950408889634f;
 
 struct FwdMaps { CUtensorMap q, k, v, h, cs; };   // cs: the per-chunk state buffer (2-D, rows of DH)
 
-// Developer aid: -DMLSTM_TIMELINE makes CTA 0 dump clock64() stamps of every phase of every
-// chunk (compute thread 0 and the issuer) into p.workspace (tests/gpu_tools/timeline.py).
-#ifdef MLSTM_TIMELINE
-#define TL_STAMP(k) do { if (blockIdx.x == 0 && threadIdx.x == 0) tl_buf[(c) * 32 + (k)] = clock64(); \
-                          if (blockIdx.x == 0 && threadIdx.x == CT) tl_buf[(c) * 32 + 16 + (k)] = clock64(); } while (0)
-#define TL_HEAD(k) do { if (blockIdx.x == 0 && (threadIdx.x == 0 || threadIdx.x == CT)) \
-    reinterpret_cast<long long*>(p.workspace)[1024 + (threadIdx.x == 0 ? 0 : 8) + (k)] = clock64(); } while (0)
-#else
-#define TL_STAMP(k) do { } while (0)
-#define TL_HEAD(k) do { } while (0)
-#endif
-
 struct alignas(16) GateBuf {       // indexed by tile row
   float u2[L];         // u * log2e + log2(scale)   (exponent of P, scale folded in)
   float M2[L];         // M * log2e
@@ -60,23 +53,6 @@ struct alignas(16) GateBuf {       // indexed by tile row
   float decay;         // exp(m_prev - M_L)
   float m_next;        // g + M_L
   float pad[2];
-};
-
-template <int DH>
-struct Smem {
-  static constexpr int KT = DH / 64;               // 64-wide tiles per operand
-  static constexpr int TILE_C = DH * 128;          // bytes of one [DH rows][64] Cb tile
-  alignas(1024) uint8_t q[KT * TILE];
-  alignas(1024) uint8_t k[2][KT * TILE];           // double buffered: K(c+1) streams in during chunk c
-  alignas(1024) uint8_t v[KT * TILE];
-  alignas(1024) uint8_t cb[KT * TILE_C];           // bf16 C, MN-major [dk][dv]
-  alignas(1024) uint8_t ones[2048];                // bf16 1.0 (B operand of n += Kbar^T 1)
-  GateBuf g[3];                                    // ring: chunk c uses g[c % 3]
-  float n_prev[DH];
-  float part_qn[4][L];                             // per column-block partials of q . n_prev
-  float part_rs[4][L];                             // per column-block partials of the row sums of P
-  uint64_t bar_q, bar_k[2], bar_v, bar_m1, bar_kv, bar_m2;
-  uint32_t tmem_base;
 };
 
 __device__ __forceinline__ float ex2(float x) {
@@ -155,430 +131,6 @@ __device__ __forceinline__ void compute_gates(GateBuf& G, const mlstm_params& p,
   __syncwarp();
 }
 
-template <int DH>
-__global__ void __launch_bounds__(NT, 1) tc_fwd_kernel(const __grid_constant__ FwdMaps maps, const mlstm_params p,
-                                                       const float scale) {
-  constexpr int KT = DH / 64;
-  constexpr int TILE_C = Smem<DH>::TILE_C;
-  constexpr int NB = DH / 32;                                // 32-column blocks of a DH-wide matrix
-  constexpr uint32_t A_LBO_STATE = (DH == 128) ? TILE : 0;  // DH=64: the 2nd 64-row M block aliases the 1st
-  extern __shared__ __align__(1024) uint8_t smem_raw[];   // 128B-swizzled tiles need 1024-byte alignment
-  Smem<DH>& sm = *reinterpret_cast<Smem<DH>*>(smem_raw);       // no pointer arithmetic: keeps the shared address space (LDS/STS)
-  if ((smem_u32(smem_raw) & 1023u) != 0) __trap();
-  TL_HEAD(0);
-
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const bool compute = tid < CT;
-  const bool issuer = tid == CT;       // lane 0 of the control warp
-  const bool gatew = tid >= GT0;       // gate warps
-  const int rg = warp & 3;             // row group: tile rows / TMEM lanes 32*rg .. 32*rg+31
-  const int cq = compute ? (warp >> 2) : 4;   // column block: columns 32*cq .. 32*cq+31 (4 = none)
-  const int row = rg * 32 + lane;      // this thread's tile row
-  const int bh = blockIdx.x, b = bh / p.NH, h = bh % p.NH;
-  const int S = p.S, NC = (S + L - 1) / L;
-  const bool has_init = p.c_initial != nullptr;
-  const bool rev = p.reverse != 0;
-  // per-chunk entry states for the backward (only when a backward will follow: n_row given)
-  const bool save_states = p.states != nullptr && p.n_row != nullptr;
-  const tc::StateLayout slay(p.B, p.NH, S, DH);
-  __nv_bfloat16* Cs_g = reinterpret_cast<__nv_bfloat16*>(reinterpret_cast<uint8_t*>(p.states) + slay.cs_off) + (size_t)bh * NC * DH * DH;
-  float* ns_g = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(p.states) + slay.ns_off) + (size_t)bh * NC * DH;
-  float* ms_g = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(p.states) + slay.ms_off) + (size_t)bh * NC;
-
-  if (issuer) {
-    tma_prefetch_desc(&maps.q); tma_prefetch_desc(&maps.k); tma_prefetch_desc(&maps.v); tma_prefetch_desc(&maps.h);
-    mbar_init(&sm.bar_q, 1); mbar_init(&sm.bar_k[0], 1); mbar_init(&sm.bar_k[1], 1); mbar_init(&sm.bar_v, 1);
-    mbar_init(&sm.bar_m1, 2); mbar_init(&sm.bar_kv, 2); mbar_init(&sm.bar_m2, 1);
-    fence_mbar_init();
-  }
-  if (warp == 0) tmem_alloc(&sm.tmem_base, 512);
-  // ones tile; zero Cb / n_prev when there is no initial state
-  for (int e = tid; e < 2048 / 4; e += NT) reinterpret_cast<uint32_t*>(sm.ones)[e] = 0x3F803F80u;
-  if (!has_init) {
-    for (int e = tid; e < KT * TILE_C / 16; e += NT) reinterpret_cast<uint4*>(sm.cb)[e] = make_uint4(0, 0, 0, 0);
-    for (int e = tid; e < DH; e += NT) sm.n_prev[e] = 0.f;
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tm = sm.tmem_base;
-  const uint32_t tS = tm, tG = tm + 128, tC = tm + 128 + DH, tN = tm + 128 + 2 * DH;
-  const uint32_t tP = tm + 448;   // P as packed bf16 (64 columns): the A operand of MMA2, read from TMEM
-  const uint32_t lane_sel = (uint32_t)(rg * 32) << 16;
-
-  auto tok0_of = [&](int c) { return (rev ? (NC - 1 - c) : c) * L; };
-  auto issue_loads = [&](uint8_t* dst, const CUtensorMap* map, uint64_t* bar, int c) {
-    mbar_arrive_expect_tx(bar, KT * TILE);
-    for (int kt = 0; kt < KT; ++kt) tma_load_4d(dst + kt * TILE, map, bar, kt * 64, tok0_of(c), h, b);
-  };
-  // UMMA shared-memory descriptors are loop invariant: build them once, advance per k-step by
-  // adding a constant to the start-address field (issue cost: a couple of instructions per MMA).
-  const uint64_t dQ = make_sdesc(smem_u32(sm.q), 16, 1024);
-  const uint64_t dCbmn = make_sdesc(smem_u32(sm.cb), TILE_C, 1024), dVmn = make_sdesc(smem_u32(sm.v), TILE, 1024);
-  const uint64_t dOnes = make_sdesc(smem_u32(sm.ones), 1024, 1024);
-  const uint64_t dKk0 = make_sdesc(smem_u32(sm.k[0]), 16, 1024), dKmn0 = make_sdesc(smem_u32(sm.k[0]), A_LBO_STATE, 1024);
-  constexpr uint64_t KBUF_STEP = (uint64_t)(KT * TILE) >> 4;     // descriptor distance between the two K buffers
-  auto kstep = [](int ks) { return (uint64_t)((((ks >> 2) * TILE) + (ks & 3) * 32) >> 4); };   // K-major advance
-  auto mnstep = [](int ks) { return (uint64_t)((ks * 2048) >> 4); };                             // MN-major advance
-  // MMA1 of chunk c, one product per call (each arrives once on bar_m1): part 0: S = Q K^T, part 1: G = Q Cb.  A single lane
-  // issues at ~100 cycles per MMA (register-to-uniform waterfall in front of each tcgen05.mma) while the tensor pipe needs
-  // 50-70, so the two independent products go out from two lanes (control lane; lane 0 of compute warp 1).
-  auto issue_mma1 = [&](int c, int part) {
-    if (part == 0) {
-      const uint64_t dKk = dKk0 + (c & 1) * KBUF_STEP;
-      constexpr uint32_t idS = make_idesc_bf16(128, 128, 0, 0);
-#pragma unroll
-      for (int ks = 0; ks < DH / 16; ++ks) umma_bf16_ss(tS, dQ + kstep(ks), dKk + kstep(ks), idS, ks > 0);
-    } else {
-      constexpr uint32_t idG = make_idesc_bf16(128, DH, 0, 1);
-#pragma unroll
-      for (int ks = 0; ks < DH / 16; ++ks) umma_bf16_ss(tG, dQ + kstep(ks), dCbmn + mnstep(ks), idG, ks > 0);
-    }
-    umma_commit(&sm.bar_m1);
-  };
-
-  // ---- prologue: first loads, gates of chunks 0 and 1, initial state -----------------------
-  TL_HEAD(1);
-  if (issuer) {
-    issue_loads(sm.q, &maps.q, &sm.bar_q, 0);
-    issue_loads(sm.k[0], &maps.k, &sm.bar_k[0], 0);
-    issue_loads(sm.v, &maps.v, &sm.bar_v, 0);
-  }
-  if (gatew) {
-    compute_gates<DH>(sm.g[0], p, b, h, 0, lane, p.m_initial ? p.m_initial[bh] : 0.f, scale);
-    // chunk 1's gates need chunk 0's m_next (serial) but nobody reads them before the state pass of chunk 0:
-    // they are computed during chunk 0 (barrier 6 below) instead of lengthening the prologue
-  }
-  __syncthreads();
-  TL_HEAD(2);
-
-  if (has_init) {  // TMEM C <- decay_0 * C_0 ; Cb <- bf16(C_0) ; n likewise  (thread: state row `row`, block cq)
-    const float d0 = sm.g[0].decay;
-    if (row < DH && cq < NB) {
-      const float* crow = p.c_initial + ((int64_t)bh * DH + row) * DH + cq * 32;
-      float r[32];
-#pragma unroll
-      for (int x = 0; x < 32; ++x) r[x] = crow[x];
-#pragma unroll
-      for (int x = 0; x < 32; x += 8) {
-        const int dv = cq * 32 + x;
-        *reinterpret_cast<uint4*>(sm.cb + (dv >> 6) * TILE_C + swz128(row, dv & 63)) =
-            make_uint4(pack_bf16x2(r[x], r[x + 1]), pack_bf16x2(r[x + 2], r[x + 3]), pack_bf16x2(r[x + 4], r[x + 5]),
-                       pack_bf16x2(r[x + 6], r[x + 7]));
-      }
-#pragma unroll
-      for (int x = 0; x < 32; ++x) r[x] *= d0;
-      tmem_st32(tC + lane_sel + cq * 32, r);
-      if (cq == 0) {
-        const float n0 = p.n_initial[(int64_t)bh * DH + row];
-        sm.n_prev[row] = n0;
-#pragma unroll
-        for (int x = 0; x < 32; ++x) r[x] = n0 * d0;
-        tmem_st32(tN + lane_sel, r);   // tN occupies 16 columns; the next 16 are unused scratch
-      }
-      tmem_st_wait();
-    }
-    fence_proxy_async_smem();
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-  }
-  if (save_states && row < DH && cq < NB) {   // entry state of chunk 0
-    uint32_t pk[16];
-    const float* crow = has_init ? p.c_initial + ((int64_t)bh * DH + row) * DH + cq * 32 : nullptr;
-#pragma unroll
-    for (int x = 0; x < 32; x += 2) pk[x / 2] = has_init ? pack_bf16x2(crow[x], crow[x + 1]) : 0u;
-    tc::store_row32(Cs_g + (size_t)row * DH + cq * 32, pk);
-    if (cq == 0) ns_g[row] = has_init ? p.n_initial[(int64_t)bh * DH + row] : 0.f;
-  }
-  if (save_states && issuer) ms_g[0] = (p.m_initial && !p.gate_mode) ? p.m_initial[bh] : 0.f;
-  if (issuer) {   // MMA1 of chunk 0 (later chunks: issued while the previous epilogue finishes)
-    mbar_wait(&sm.bar_q, 0);
-    mbar_wait(&sm.bar_k[0], 0);
-    tc_fence_after();
-    issue_mma1(0, 0);
-    issue_mma1(0, 1);
-  }
-
-#ifdef MLSTM_TIMELINE
-  long long* tl_buf = reinterpret_cast<long long*>(p.workspace);
-#endif
-  TL_HEAD(3);
-  for (int c = 0; c < NC; ++c) {
-    TL_STAMP(0);
-    const uint32_t ph = c & 1;
-    const bool last = (c + 1 == NC);
-    if (gatew) {
-      // two chunks ahead, into the ring slot chunk c-1 just released
-      if (c == 0 && NC > 1) {
-        compute_gates<DH>(sm.g[1], p, b, h, 1, lane, sm.g[0].m_next, scale);
-        named_sync(6, GT0);   // with the compute warps, ahead of chunk 0's state pass (first reader: decay of chunk 1)
-      }
-      if (c + 2 < NC) compute_gates<DH>(sm.g[(c + 2) % 3], p, b, h, c + 2, lane, sm.g[(c + 1) % 3].m_next, scale);
-      __syncthreads();   // the end-of-chunk barrier is the only one the gate warp takes part in
-      continue;
-    }
-    GateBuf& G = sm.g[c % 3];
-    const int tok0 = tok0_of(c);
-    uint8_t* sk = sm.k[c & 1];
-    // the state leaving the last chunk is only needed when the caller asked for it: otherwise the last step skips the K
-    // rescale, the state MMA and the state pass
-    const bool do_state = !last || p.c_last != nullptr;
-
-    // ---- top: K(c+1) streams into the other buffer (once the h(c-1) staged there has been read)
-    if (issuer && !last) {
-      tma_store_wait_read<0>();
-      issue_loads(sm.k[(c + 1) & 1], &maps.k, &sm.bar_k[(c + 1) & 1], c + 1);
-    }
-    mbar_wait(&sm.bar_q, ph);
-    mbar_wait(&sm.bar_k[c & 1], (c >> 1) & 1);
-    TL_STAMP(1);
-    // partial q . n_prev in the MMA1 shadow: this thread: row `row`, dk in [32 cq, 32 cq + 32)
-    if (cq < NB) {
-      float qn = 0.f;
-#pragma unroll
-      for (int x = 0; x < 32; x += 8) {
-        const int col = cq * 32 + x;
-        const uint4 w = *reinterpret_cast<const uint4*>(sm.q + (col >> 6) * TILE + swz128(row, col & 63));
-        const float4 n0 = *reinterpret_cast<const float4*>(&sm.n_prev[col]);
-        const float4 n1 = *reinterpret_cast<const float4*>(&sm.n_prev[col + 4]);
-        const __nv_bfloat162* qq = reinterpret_cast<const __nv_bfloat162*>(&w);
-        float2 a = __bfloat1622float2(qq[0]), bq = __bfloat1622float2(qq[1]), cq_ = __bfloat1622float2(qq[2]),
-               dq = __bfloat1622float2(qq[3]);
-        qn += a.x * n0.x + a.y * n0.y + bq.x * n0.z + bq.y * n0.w + cq_.x * n1.x + cq_.y * n1.y + dq.x * n1.z + dq.y * n1.w;
-      }
-      sm.part_qn[cq][row] = qn;
-    } else if (compute) {
-      sm.part_qn[cq][row] = 0.f;
-    }
-    TL_STAMP(2);
-    mbar_wait(&sm.bar_m1, ph);     // S(c) and G(c) are in TMEM
-    tc_fence_after();
-    TL_STAMP(3);
-
-    // ---- P = S * exp2(u2_j - M2_t), causal: one 32x32 block per warp; partial row sums ----
-    if (compute) {
-      const float M2t = G.M2[row];
-      // forward: keys j <= t ; reverse: keys j >= t   (tile rows)
-      const bool full = rev ? (cq > rg) : (cq < rg);
-      const bool diag = (cq == rg);
-      uint32_t packed[16];
-      float rowsum = 0.f;
-      if (full || diag) {
-        float s[32];
-        tmem_ld32(tS + lane_sel + cq * 32, s);
-        const uint32_t cbits = causal_bits(full, !rev, lane);
-        tmem_ld_wait();
-#pragma unroll
-        for (int x = 0; x < 32; x += 4) {
-          const float4 u4 = *reinterpret_cast<const float4*>(&G.u2[cq * 32 + x]);
-          const float uu[4] = {u4.x, u4.y, u4.z, u4.w};
-          float pv[4];
-#pragma unroll
-          for (int e = 0; e < 4; ++e) {
-            const bool keep = (cbits >> (x + e)) & 1u;
-            pv[e] = keep ? s[x + e] * ex2(uu[e] - M2t) : 0.f;
-            rowsum += pv[e];
-          }
-          packed[x / 2] = pack_bf16x2(pv[0], pv[1]);
-          packed[x / 2 + 1] = pack_bf16x2(pv[2], pv[3]);
-        }
-      } else {
-#pragma unroll
-        for (int x = 0; x < 16; ++x) packed[x] = 0u;
-      }
-      sm.part_rs[cq][row] = rowsum;
-      // P stays on the tensor-core side: no shared-memory round trip, and MMA2 reads only V from smem
-      // (an SS-form MMA at this shape is shared-memory-read bound and starves the SIMT work in its shadow)
-      tmem_st16(tP + lane_sel + cq * 16, packed);
-      tmem_st_wait();
-    }
-    TL_STAMP(4);
-    tc_fence_before();
-    named_sync(2, GT0);
-    TL_STAMP(5);
-
-    // ---- MMA2: H = P V (into the S columns); Q(c+1) prefetch (Q(c) is dead) ----------------
-    if (issuer) {
-      if (!last) issue_loads(sm.q, &maps.q, &sm.bar_q, c + 1);
-      mbar_wait(&sm.bar_v, ph);
-      tc_fence_after();
-      constexpr uint32_t idH = make_idesc_bf16(128, DH, 0, 1);
-#pragma unroll
-      for (int ks = 0; ks < L / 16; ++ks) umma_bf16_ts(tS, tP + ks * 8, dVmn + mnstep(ks), idH, ks > 0);
-      umma_commit(&sm.bar_m2);
-    }
-    // ---- in the MMA2 shadow: normaliser, n-state partials, Kbar = kw * K in place ------------
-    const float wq = G.wq[row];
-    const float mrow = G.mrow[row];
-    const float nr = (sm.part_rs[0][row] + sm.part_rs[1][row] + sm.part_rs[2][row] + sm.part_rs[3][row]) +
-                     wq * (sm.part_qn[0][row] + sm.part_qn[1][row] + sm.part_qn[2][row] + sm.part_qn[3][row]);
-    const float inv = 1.f / (fmaxf(fabsf(nr), __expf(-mrow)) + p.eps);   // backends.py:249-252
-    if (cq == 0) {
-      const int tok = tok0 + row;
-      if (p.n_row && tok < S) {
-        p.n_row[(int64_t)bh * S + tok] = nr;
-        p.m_row[(int64_t)bh * S + tok] = mrow;
-      }
-    }
-#pragma unroll
-    for (int it = 0; it < ((compute && do_state) ? KT * TILE / 16 / CT : 0); ++it) {
-      const uint32_t o = (uint32_t)(tid + it * CT) * 16u;
-      const int krow = (o >> 7) & (L - 1);
-      const float s = G.kw[krow];
-      uint4 w = *reinterpret_cast<uint4*>(sk + o);
-      __nv_bfloat162* kk = reinterpret_cast<__nv_bfloat162*>(&w);
-#pragma unroll
-      for (int e = 0; e < 4; ++e) {
-        float2 f2 = __bfloat1622float2(kk[e]);
-        kk[e] = __floats2bfloat162_rn(f2.x * s, f2.y * s);
-      }
-      *reinterpret_cast<uint4*>(sk + o) = w;
-    }
-    TL_STAMP(6);
-    fence_proxy_async_smem();
-    named_sync(2, GT0);
-    TL_STAMP(7);
-
-    // ---- state MMA: C += Kbar^T V ------------------------------------------------------------
-    if (issuer && do_state) {
-      tc_fence_after();
-      const uint64_t dKmn = dKmn0 + (c & 1) * KBUF_STEP;
-      constexpr uint32_t idC = make_idesc_bf16(128, DH, 1, 1);
-      const uint32_t acc0 = (c > 0 || has_init) ? 1u : 0u;
-#pragma unroll
-      for (int ks = 0; ks < L / 16; ++ks) umma_bf16_ss(tC, dKmn + mnstep(ks), dVmn + mnstep(ks), idC, (ks > 0) ? 1u : acc0);
-      umma_commit(&sm.bar_kv);
-    }
-    if (tid == 32 && do_state) {   // n += Kbar^T 1 from a second lane (lane 0 of compute warp 1); two arrivals complete bar_kv
-      tc_fence_after();
-      const uint64_t dKmn = dKmn0 + (c & 1) * KBUF_STEP;
-      constexpr uint32_t idN = make_idesc_bf16(128, 16, 1, 1);
-      const uint32_t acc0 = (c > 0 || has_init) ? 1u : 0u;
-#pragma unroll
-      for (int ks = 0; ks < L / 16; ++ks) umma_bf16_ss(tN, dKmn + mnstep(ks), dOnes, idN, (ks > 0) ? 1u : acc0);
-      umma_commit(&sm.bar_kv);
-    }
-    mbar_wait(&sm.bar_m2, ph);
-    tc_fence_after();
-    TL_STAMP(8);
-
-    // ---- epilogue part 1 (in the state-MMA shadow): h = (H + wq G) / N, packed bf16 in registers
-    uint32_t hpk[16];
-    if (cq < NB) {
-      float hi[32], gg[32];
-      tmem_ld32(tS + lane_sel + cq * 32, hi);
-      tmem_ld32(tG + lane_sel + cq * 32, gg);
-      tmem_ld_wait();
-#pragma unroll
-      for (int x = 0; x < 32; x += 2)
-        hpk[x / 2] = pack_bf16x2((hi[x] + wq * gg[x]) * inv, (hi[x + 1] + wq * gg[x + 1]) * inv);
-    }
-    TL_STAMP(9);
-    if (do_state) {
-      mbar_wait(&sm.bar_kv, ph);   // state update complete: C final, Kbar and V dead
-      tc_fence_after();
-    }
-    TL_STAMP(10);
-    if (issuer && !last) issue_loads(sm.v, &maps.v, &sm.bar_v, c + 1);
-
-    // ---- state pass: Cb <- bf16(C); C <- decay_next C (state row `row`, block cq); n in smem ----
-    if (c == 0 && NC > 1 && compute) named_sync(6, GT0);   // chunk 1's gates (gate warp, computed during this chunk) are complete
-    const float dnext = last ? 1.f : sm.g[(c + 1) % 3].decay;
-    if (cq < NB) {
-      if (row < DH && do_state) {
-        float r[32];
-        tmem_ld32(tC + lane_sel + cq * 32, r);
-        tmem_ld_wait();
-        if (last && p.c_last) {
-          float* dst = p.c_last + ((int64_t)bh * DH + row) * DH + cq * 32;
-#pragma unroll
-          for (int x = 0; x < 32; x += 4) *reinterpret_cast<float4*>(dst + x) = make_float4(r[x], r[x + 1], r[x + 2], r[x + 3]);
-        }
-        {
-          uint32_t pk[16];
-#pragma unroll
-          for (int x = 0; x < 32; x += 2) pk[x / 2] = pack_bf16x2(r[x], r[x + 1]);
-#pragma unroll
-          for (int x = 0; x < 4; ++x) {
-            const int dv = cq * 32 + x * 8;
-            *reinterpret_cast<uint4*>(sm.cb + (dv >> 6) * TILE_C + swz128(row, dv & 63)) =
-                make_uint4(pk[4 * x], pk[4 * x + 1], pk[4 * x + 2], pk[4 * x + 3]);
-          }
-        }
-        if (!last) {
-#pragma unroll
-          for (int x = 0; x < 32; ++x) r[x] *= dnext;
-          tmem_st32(tC + lane_sel + cq * 32, r);
-        }
-        if (cq == 0) {
-          float rn[16];
-          tmem_ld16(tN + lane_sel, rn);
-          tmem_ld_wait();
-          sm.n_prev[row] = rn[0];
-          if (save_states && !last) ns_g[(size_t)(c + 1) * DH + row] = rn[0];
-          if (last && p.n_last) p.n_last[(int64_t)bh * DH + row] = rn[0];
-          if (!last) {
-#pragma unroll
-            for (int x = 0; x < 32; ++x) r[x] = rn[0] * dnext;
-            tmem_st32(tN + lane_sel, r);
-          }
-        }
-        if (!last) tmem_st_wait();
-      }
-      // ---- epilogue part 2: stage h in the (now dead) K buffer of this chunk for the TMA store ----
-#pragma unroll
-      for (int x = 0; x < 4; ++x) {
-        const int dv = cq * 32 + x * 8;
-        *reinterpret_cast<uint4*>(sk + (dv >> 6) * TILE + swz128(row, dv & 63)) =
-            make_uint4(hpk[4 * x], hpk[4 * x + 1], hpk[4 * x + 2], hpk[4 * x + 3]);
-      }
-    }
-    if (last && p.m_last && issuer) p.m_last[bh] = G.m_next;
-    if (save_states && !last && issuer) ms_g[c + 1] = G.m_next;
-    TL_STAMP(11);
-    fence_proxy_async_smem();
-    tc_fence_before();
-    __syncthreads();   // end of chunk: everybody, including the gate warp
-    TL_STAMP(12);
-    if (issuer) {
-      for (int kt = 0; kt < KT; ++kt) tma_store_4d(&maps.h, sk + kt * TILE, kt * 64, tok0, h, b);
-      if (save_states && !last)   // entry state of chunk c+1 = the bf16 C tile just written (read again by the next state pass only)
-        for (int kt = 0; kt < KT; ++kt) tma_store_2d(&maps.cs, sm.cb + kt * TILE_C, kt * 64, (bh * NC + c + 1) * DH);
-      tma_store_commit();
-      if (!last) {   // MMA1 of the next chunk, S part
-        mbar_wait(&sm.bar_q, ph ^ 1);
-        mbar_wait(&sm.bar_k[(c + 1) & 1], ((c + 1) >> 1) & 1);
-        tc_fence_after();
-        issue_mma1(c + 1, 0);
-      }
-    }
-    if (tid == 32 && !last) {   // G part (Cb was refreshed by the state pass above)
-      mbar_wait(&sm.bar_q, ph ^ 1);
-      tc_fence_after();
-      issue_mma1(c + 1, 1);
-    }
-  }
-
-  TL_HEAD(4);
-  if (issuer) tma_store_wait_all<0>();
-  tc_fence_before();
-  __syncthreads();
-  TL_HEAD(5);
-  if (warp == 0) tmem_dealloc(tm, 512);
-}
-
-
-// =====================================================================================================================
-// Warp-specialised variant of the walk: the 16 compute warps split into two groups that work on the two dependency
-// chains of a chunk CONCURRENTLY instead of alternating through CTA-wide barriers:
-//   group A (warps 0-7)   the score chain    wait S -> P = S * exp2(u - M) -> [MMA2 H = P V] -> h = (H + w G) / N
-//   group B (warps 8-15)  the state chain    q . n_prev -> Kbar = kw K -> [state MMA] -> Cb <- bf16(C), C <- decay C, n
-// A warp owns tile rows 32*(w%4)..+31 (its TMEM lane quadrant) and one half of the columns (two 32-column blocks).  The
-// control lane polls the two hand-offs (P written, Kbar written) and issues MMA2 / the state MMA in whichever order they
-// become ready; one CTA-wide barrier per chunk remains (gate ring, G of the next chunk after the state pass).  h is staged
-// in its own tile (the K buffer is no longer available: the state chain may still be reading it).
-// =====================================================================================================================
 template <int DH>
 struct SmemWS {
   static constexpr int KT = DH / 64;
@@ -675,7 +227,7 @@ __global__ void __launch_bounds__(NT, 1) tc_fwd_ws_kernel(const __grid_constant_
     umma_commit(part == 0 ? &sm.bar_s : &sm.bar_g);
   };
 
-  // ---- prologue (as in the one-group kernel): first loads, gates of chunk 0, initial state ------------------------------
+  // ---- prologue: first loads, gates of chunk 0, initial state ------------------------------------------------------
   if (issuer) {
     issue_loads(sm.q, &maps.q, &sm.bar_q, 0);
     issue_loads(sm.k[0], &maps.k, &sm.bar_k[0], 0);
@@ -1011,17 +563,13 @@ int launch_fwd(const mlstm_params& p, cudaStream_t st) {
     set_error("cuTensorMapEncodeTiled failed (%d): pointers must be 16-byte aligned, strides multiples of 8 elements", r);
     return r == -1 ? MLSTM_ERR_NO_DEVICE : MLSTM_ERR_INVALID_ARG;
   }
-  // warp-specialised walk by default (cfg3 forward 72.4 -> 67 us, cfg2 25.2 -> 24 us); MLSTM_FWD_WS=0 selects the one-group kernel
-  static const bool ws = !(getenv("MLSTM_FWD_WS") != nullptr && getenv("MLSTM_FWD_WS")[0] == '0');
-  const size_t smem = ws ? sizeof(SmemWS<DH>) + 1024 : sizeof(Smem<DH>) + 1024;
-  const void* kern = ws ? reinterpret_cast<const void*>(tc_fwd_ws_kernel<DH>) : reinterpret_cast<const void*>(tc_fwd_kernel<DH>);
-  cudaError_t e = set_max_smem_once(kern, smem);
+  const size_t smem = sizeof(SmemWS<DH>) + 1024;
+  cudaError_t e = set_max_smem_once(reinterpret_cast<const void*>(tc_fwd_ws_kernel<DH>), smem);
   if (e != cudaSuccess) {
     set_error("cudaFuncSetAttribute(tc_fwd, %zu B): %s", smem, cudaGetErrorString(e));
     return MLSTM_ERR_CUDA;
   }
-  if (ws) tc_fwd_ws_kernel<DH><<<dim3(p.B * p.NH), dim3(NT), smem, st>>>(maps, p, resolve_scale(p));
-  else tc_fwd_kernel<DH><<<dim3(p.B * p.NH), dim3(NT), smem, st>>>(maps, p, resolve_scale(p));
+  tc_fwd_ws_kernel<DH><<<dim3(p.B * p.NH), dim3(NT), smem, st>>>(maps, p, resolve_scale(p));
   count_launch();
   e = cudaGetLastError();
   if (e != cudaSuccess) {

@@ -26,9 +26,6 @@ __device__ __forceinline__ float ex2(float x) {
 __device__ __forceinline__ void named_sync(int id, int nthreads) {
   asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
 }
-__device__ __forceinline__ void named_arrive(int id, int nthreads) {   // arrive without waiting (producer side)
-  asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
-}
 // log(sigmoid(x)) with fast intrinsics (abs error < 1e-7, enough for the bf16 path)
 __device__ __forceinline__ float log_sigmoid_fast(float x) { return fminf(x, 0.f) - __logf(1.f + __expf(-fabsf(x))); }
 
@@ -233,19 +230,6 @@ __device__ __forceinline__ void store_row32(__nv_bfloat16* dst, const uint32_t (
 #pragma unroll
   for (int x = 0; x < 4; ++x)
     *reinterpret_cast<uint4*>(dst + x * 8) = make_uint4(pk[4 * x], pk[4 * x + 1], pk[4 * x + 2], pk[4 * x + 3]);
-}
-__device__ __forceinline__ void load_row32(const __nv_bfloat16* src, float (&out)[32]) {
-#pragma unroll
-  for (int x = 0; x < 4; ++x) {
-    const uint4 w = *reinterpret_cast<const uint4*>(src + x * 8);
-    const __nv_bfloat162* qq = reinterpret_cast<const __nv_bfloat162*>(&w);
-#pragma unroll
-    for (int e = 0; e < 4; ++e) {
-      float2 f2 = __bfloat1622float2(qq[e]);
-      out[x * 8 + 2 * e] = f2.x;
-      out[x * 8 + 2 * e + 1] = f2.y;
-    }
-  }
 }
 
 // 2-D tensor map over a [rows][DH] bf16 matrix stack (the Cs / dCs workspace): dims (DH, rows_total)
