@@ -73,7 +73,7 @@ class MultiHeadLayerNorm(nn.Module):
 
 def _fused_gates_ok(dim: int) -> bool:
     from . import ops
-    return ops.gates_supported(dim)
+    return ops.gates_supported(int(dim))
 
 
 class MatrixLSTMCell(nn.Module):
@@ -135,8 +135,7 @@ class MatrixLSTMCell(nn.Module):
             raise ValueError("All input tensors (q, k, v) must be on the same device.")
         backend = self.gpu_backend if self.training else self.gpu_backend_infer
         with torch.autograd.profiler.record_function("ViLLayer::mlstm_cell"):
-            # (under torch.compile the cell goes through the registered custom op and the gate projection stays with the compiler)
-            if q.is_cuda and getattr(self, "fused_gates", True) and not torch.compiler.is_compiling() and _fused_gates_ok(H):
+            if q.is_cuda and getattr(self, "fused_gates", True) and _fused_gates_ok(H):
                 # hand-written gate projection fused with the cell into one autograd node
                 h = backend.fused_cell(q, k, v, self.igate, self.fgate, self.num_heads, reverse=reverse)
             else:

@@ -105,19 +105,24 @@ def kernel_family(q: torch.Tensor, v: torch.Tensor) -> str:
     return name.decode() if name else "none"
 
 
-def _alloc_states(lib, p, dev):
-    """Per-chunk entry-state buffer of the tcgen05 family (None for SIMT); attaches it to p."""
-    with torch.cuda.device(dev):   # size and variant queries see the device the launch will see
-        need = lib.mlstm_b200_state_bytes(C.byref(p))
+def _alloc_states(lib, p, dev, nbytes=None):
+    """Per-chunk entry-state buffer of the tcgen05 family (None for SIMT); attaches it to p.  ``nbytes``: a size the caller
+    chose (the custom ops, ``_states_numel``), zero-filled so that the bytes the kernels leave unwritten (alignment padding)
+    do not differ from call to call; the library checks that it suffices."""
+    if nbytes is None:
+        with torch.cuda.device(dev):   # size and variant queries see the device the launch will see
+            need = lib.mlstm_b200_state_bytes(C.byref(p))
+    else:
+        need = nbytes
     if not need:
         return None
-    states = torch.empty(need, dtype=torch.uint8, device=dev)
+    states = (torch.empty if nbytes is None else torch.zeros)(need, dtype=torch.uint8, device=dev)
     p.states, p.states_bytes = states.data_ptr(), need
     return states
 
 
 def mlstm_fwd_raw(q, k, v, i, f, c_initial=None, n_initial=None, m_initial=None, *, eps=1e-6, chunk_size=64,
-                  reverse=False, save_rows=True, return_last_states=False, qk_scale=None, gate_mode=0):
+                  reverse=False, save_rows=True, return_last_states=False, qk_scale=None, gate_mode=0, states_bytes=None):
     """One forward launch through the C ABI.  Inputs must already be CUDA, fp32 or bf16
     (q,k,v same dtype), gates fp32.  Returns (h, n_row, m_row, last_states_or_None, chunk_states)."""
     lib = _lib.load()
@@ -140,7 +145,7 @@ def mlstm_fwd_raw(q, k, v, i, f, c_initial=None, n_initial=None, m_initial=None,
     p.n_row, p.m_row = _ptr(n_row), _ptr(m_row)
     if last is not None:
         p.c_last, p.n_last, p.m_last = (_ptr(t) for t in last)
-    states = _alloc_states(lib, p, dev)
+    states = _alloc_states(lib, p, dev, states_bytes)
     with torch.cuda.device(dev):
         rc = lib.mlstm_b200_fwd(C.byref(p), _stream())
     if rc:
@@ -219,8 +224,17 @@ class _MLSTMCellFn(torch.autograd.Function):
 # cell (the reference compiles its model in debug.py:13).  ``mlstm`` takes this route while torch.compile is tracing and
 # the plain autograd.Function otherwise (same kernels, less dispatch overhead per call in eager mode).
 # ---------------------------------------------------------------------------------------------
-def _states_numel(B, NH, S, DK, DV, dtype, save_rows: bool) -> int:
-    """Bytes of the chunk-state buffer for these shapes (a host-side query: no device pointers involved)."""
+def _states_numel(B, NH, S, DK, DV, dtype):
+    """Bytes of the chunk-state buffer the custom ops allocate and their fakes declare: B times what one batch row needs
+    with a backward following.  That bounds the library's need at every batch size, variant and forward-only call
+    (tests/test_gpu_compile.py), and stays a plain function of a symbolic batch, so a dynamic batch traces into one graph
+    (the other sizes specialise)."""
+    return B * _state_bytes(1, int(NH), int(S), int(DK), int(DV), dtype, True)
+
+
+@torch.compiler.assume_constant_result
+def _state_bytes(B: int, NH: int, S: int, DK: int, DV: int, dtype: torch.dtype, save_rows: bool) -> int:
+    """``mlstm_b200_state_bytes`` for these shapes (a host-side query: no device pointers involved)."""
     p = Params()
     p.abi_version = _lib.ABI_VERSION
     p.B, p.NH, p.S, p.DHQK, p.DHV = B, NH, S, DK, DV
@@ -234,11 +248,11 @@ def _states_numel(B, NH, S, DK, DV, dtype, save_rows: bool) -> int:
 def _mlstm_fwd_op(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, i: torch.Tensor, f: torch.Tensor,
                   c_initial: Optional[torch.Tensor], n_initial: Optional[torch.Tensor], m_initial: Optional[torch.Tensor],
                   eps: float, chunk_size: int, reverse: bool, save_rows: bool, return_last_states: bool,
-                  gate_mode: int) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
+                  gate_mode: int, states_bytes: int) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
     q, k, v = _prep_act(q), _prep_act(k), _prep_act(v)
     h, n_row, m_row, last, states = mlstm_fwd_raw(q, k, v, i, f, c_initial, n_initial, m_initial, eps=eps, chunk_size=chunk_size,
                                                   reverse=reverse, save_rows=save_rows, return_last_states=return_last_states,
-                                                  gate_mode=gate_mode)
+                                                  gate_mode=gate_mode, states_bytes=states_bytes)
     e = lambda dt=torch.float32: torch.empty(0, dtype=dt, device=q.device)
     c_l, n_l, m_l = last if last is not None else (e(), e(), e())
     return (h, n_row if n_row is not None else e(), m_row if m_row is not None else e(),
@@ -246,14 +260,15 @@ def _mlstm_fwd_op(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, i: torch.Te
 
 
 @_mlstm_fwd_op.register_fake
-def _(q, k, v, i, f, c_initial, n_initial, m_initial, eps, chunk_size, reverse, save_rows, return_last_states, gate_mode):
+def _(q, k, v, i, f, c_initial, n_initial, m_initial, eps, chunk_size, reverse, save_rows, return_last_states, gate_mode,
+      states_bytes):
     B, NH, S, DK = q.shape
     DV = v.shape[-1]
     dev = q.device
     e = lambda dt=torch.float32: torch.empty(0, dtype=dt, device=dev)
     h = torch.empty((B, S, NH, DV), dtype=q.dtype, device=dev).transpose(1, 2)
     rows = (lambda: torch.empty((B, NH, S), dtype=torch.float32, device=dev)) if save_rows else e
-    states = torch.empty(_states_numel(B, NH, S, DK, DV, q.dtype, save_rows), dtype=torch.uint8, device=dev)
+    states = torch.empty(states_bytes, dtype=torch.uint8, device=dev)
     if return_last_states:
         last = (torch.empty((B, NH, DK, DV), dtype=torch.float32, device=dev), torch.empty((B, NH, DK), dtype=torch.float32, device=dev),
                 torch.empty((B, NH, 1), dtype=torch.float32, device=dev))
@@ -285,7 +300,7 @@ def _(q, k, v, i, f, h, n_row, m_row, dh, c_initial, n_initial, m_initial, state
 
 
 def _op_setup_context(ctx, inputs, output):
-    q, k, v, i, f, c0, n0, m0, eps, chunk_size, reverse, save_rows, return_last_states, gate_mode = inputs
+    q, k, v, i, f, c0, n0, m0, eps, chunk_size, reverse, save_rows, return_last_states, gate_mode, states_bytes = inputs
     h, n_row, m_row, states = output[:4]
     ctx.save_for_backward(q, k, v, i, f, h, n_row, m_row, c0, n0, m0, states)
     ctx.cfg = (eps, chunk_size, reverse, gate_mode)
@@ -298,7 +313,7 @@ def _op_backward(ctx, dh, *_unused):
     if dh is None:
         dh = torch.zeros_like(h)
     dq, dk, dv, di, df = _mlstm_bwd_op(q, k, v, i, f, h, n_row, m_row, dh, c0, n0, m0, states, eps, chunk_size, reverse, gate_mode)
-    return dq, dk, dv, di, df, None, None, None, None, None, None, None, None, None
+    return dq, dk, dv, di, df, None, None, None, None, None, None, None, None, None, None
 
 
 _mlstm_fwd_op.register_autograd(_op_backward, setup_context=_op_setup_context)
@@ -306,8 +321,10 @@ _mlstm_fwd_op.register_autograd(_op_backward, setup_context=_op_setup_context)
 
 def _mlstm_traced(q, k, v, i, f, c0, n0, m0, eps, chunk_size, reverse, return_last_states, gate_mode):
     need_grad = torch.is_grad_enabled() and any(t.requires_grad for t in (q, k, v, i, f))
+    B, NH, S, DK = q.shape
+    nbytes = _states_numel(B, NH, S, DK, v.shape[-1], q.dtype)
     h, _n, _m, _s, c_l, n_l, m_l = _mlstm_fwd_op(q, k, v, i, f, c0, n0, m0, eps, chunk_size, reverse, need_grad,
-                                                  return_last_states, gate_mode)
+                                                  return_last_states, gate_mode, nbytes)
     return (h, c_l, n_l, m_l) if return_last_states else h
 
 
@@ -366,13 +383,23 @@ def _gate_params(q3, k3, v3, w_i, b_i, w_f, b_f, NH) -> GateProjParams:
     return g
 
 
-def _rows_ok(t: torch.Tensor) -> bool:
-    """(B,S,D) tensor whose B*S rows are evenly strided (what the gate kernels stream over)."""
+def _rows_layout_ok(t: torch.Tensor) -> bool:
+    """(B,S,D) tensor whose B*S rows are evenly strided (what the gate, tail and producer kernels stream over)."""
     B, S, D = t.shape
-    return (t.stride(2) == 1 and t.stride(0) == S * t.stride(1) and t.stride(1) % 8 == 0 and D % 8 == 0
-            and t.data_ptr() % 16 == 0)
+    return t.stride(2) == 1 and t.stride(0) == S * t.stride(1) and t.stride(1) % 8 == 0 and D % 8 == 0
 
 
+def _rows_ok(t: torch.Tensor) -> bool:
+    """``_rows_layout_ok`` with a 16-byte aligned base."""
+    return _rows_layout_ok(t) and t.data_ptr() % 16 == 0
+
+
+def _aligned(t: torch.Tensor) -> bool:
+    """16-byte aligned base.  A traced tensor has no address: the custom op it reaches copies a misaligned input."""
+    return torch.compiler.is_compiling() or t.data_ptr() % 16 == 0
+
+
+@torch.compiler.assume_constant_result
 def gates_supported(D: int, ld: Optional[int] = None) -> bool:
     """Whether csrc/mlstm_gates.cu takes a cell of inner dim D (asks the library: the 8 x 3D fp32 weight tile
     must fit in shared memory, i.e. D <= 2133)."""
@@ -418,6 +445,48 @@ def gate_proj_bwd_raw(q3, k3, v3, w_i, w_f, NH, di, df, dq3, dk3, dv3, need_bias
     return dw_i, db_i, dw_f, db_f
 
 
+def _cell_rows(q3, k3, v3, rows_ok=None):
+    """q, k, v as the gate kernels stream them: evenly strided rows sharing one row stride, else dense copies of all three.
+    ``rows_ok`` decides which layouts pass (default ``_rows_ok``; while tracing, the layout half of it)."""
+    rows_ok = rows_ok or _rows_ok
+    q3, k3, v3 = (t if rows_ok(t) else t.contiguous() for t in (q3, k3, v3))
+    if q3.stride(1) != k3.stride(1) or q3.stride(1) != v3.stride(1):
+        q3, k3, v3 = q3.contiguous(), k3.contiguous(), v3.contiguous()
+    return q3, k3, v3
+
+
+def fused_cell_fwd_raw(q3, k3, v3, w_i, b_i, w_f, b_f, NH, eps, chunk_size, reverse, gate_mode, save_rows, states_bytes=None):
+    """Gate projection + cell forward launches.  q,k,v (B,S,D) as ``_cell_rows`` leaves them, gate weights fp32.
+    Returns (h, i3, f3, n_row, m_row, states): h (B,NH,S,DH) view of (B,S,NH,DH) storage, i3, f3 (B,S,NH) fp32;
+    n_row, m_row None unless ``save_rows``; states None for the SIMT family."""
+    B, S, D = q3.shape
+    i3, f3 = gate_proj_fwd_raw(q3, k3, v3, w_i, b_i, w_f, b_f, NH)
+    heads = lambda t: t.view(B, S, NH, D // NH).transpose(1, 2)
+    h, n_row, m_row, _, states = mlstm_fwd_raw(heads(q3), heads(k3), heads(v3), i3.transpose(1, 2), f3.transpose(1, 2),
+                                               eps=eps, chunk_size=chunk_size, reverse=reverse, save_rows=save_rows,
+                                               gate_mode=gate_mode, states_bytes=states_bytes)
+    return h, i3, f3, n_row, m_row, states
+
+
+def fused_cell_bwd_raw(q3, k3, v3, w_i, w_f, i3, f3, h, n_row, m_row, states, dh, NH, eps, chunk_size, reverse, gate_mode,
+                       has_bias):
+    """Cell backward, then one streaming pass that adds the gate path into dq,dk,dv in place and reduces dW, db.
+    Returns (dq3, dk3, dv3, dw_i, db_i, dw_f, db_f): dq3.. dense (B,S,D), db_* None unless ``has_bias``."""
+    B, S, D = q3.shape
+    heads = lambda t: t.view(B, S, NH, D // NH).transpose(1, 2)
+    if dh.dtype != q3.dtype:
+        dh = dh.to(q3.dtype)
+    dh = _prep_act(dh)
+    dq, dk, dv, di, df = mlstm_bwd_raw(heads(q3), heads(k3), heads(v3), i3.transpose(1, 2), f3.transpose(1, 2), h,
+                                       n_row, m_row, dh, eps=eps, chunk_size=chunk_size, reverse=reverse,
+                                       states=states, gate_mode=gate_mode)
+    # dq,dk,dv are (B,NH,S,DH) views of fresh (B,S,NH,DH) storage; di,df views of (B,S,NH) storage
+    dq3, dk3, dv3 = (t.transpose(1, 2).reshape(B, S, D) for t in (dq, dk, dv))
+    dw_i, db_i, dw_f, db_f = gate_proj_bwd_raw(q3, k3, v3, w_i, w_f, NH, di.transpose(1, 2), df.transpose(1, 2),
+                                               dq3, dk3, dv3, need_bias=has_bias)
+    return dq3, dk3, dv3, dw_i, db_i, dw_f, db_f
+
+
 class _FusedCellFn(torch.autograd.Function):
     """q,k,v (B,S,D) + gate weights -> h (B,NH,S,DH view of (B,S,NH,DH) storage).  The backward runs
     the cell's kernels, then one streaming pass that adds the gate path into dq,dk,dv in place and
@@ -425,36 +494,18 @@ class _FusedCellFn(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, q3, k3, v3, w_i, b_i, w_f, b_f, NH, eps, chunk_size, reverse, gate_mode=0):
-        B, S, D = q3.shape
-        i3, f3 = gate_proj_fwd_raw(q3, k3, v3, w_i, b_i, w_f, b_f, NH)
-        heads = lambda t: t.view(B, S, NH, D // NH).transpose(1, 2)
-        q, k, v = heads(q3), heads(k3), heads(v3)
-        i, f = i3.transpose(1, 2), f3.transpose(1, 2)
         need_grad = any(t is not None and t.requires_grad for t in (q3, k3, v3, w_i, b_i, w_f, b_f))
-        h, n_row, m_row, _, states = mlstm_fwd_raw(q, k, v, i, f, eps=eps, chunk_size=chunk_size, reverse=reverse,
-                                                   save_rows=need_grad, gate_mode=gate_mode)
+        h, i3, f3, n_row, m_row, states = fused_cell_fwd_raw(q3, k3, v3, w_i, b_i, w_f, b_f, NH, eps, chunk_size, reverse,
+                                                             gate_mode, need_grad)
         if need_grad:
             ctx.save_for_backward(q3, k3, v3, w_i, w_f, i3, f3, h, n_row, m_row, states)
-        ctx.cfg = (NH, eps, chunk_size, reverse, b_i is not None, gate_mode)
+        ctx.cfg = (NH, eps, chunk_size, reverse, gate_mode, b_i is not None)
         return h
 
     @staticmethod
     def backward(ctx, dh):
-        q3, k3, v3, w_i, w_f, i3, f3, h, n_row, m_row, states = ctx.saved_tensors
-        NH, eps, chunk_size, reverse, has_bias, gate_mode = ctx.cfg
-        B, S, D = q3.shape
-        heads = lambda t: t.view(B, S, NH, D // NH).transpose(1, 2)
-        if dh.dtype != q3.dtype:
-            dh = dh.to(q3.dtype)
-        dh = _prep_act(dh)
-        dq, dk, dv, di, df = mlstm_bwd_raw(heads(q3), heads(k3), heads(v3), i3.transpose(1, 2), f3.transpose(1, 2), h,
-                                           n_row, m_row, dh, eps=eps, chunk_size=chunk_size, reverse=reverse,
-                                           states=states, gate_mode=gate_mode)
-        # dq,dk,dv are (B,NH,S,DH) views of fresh (B,S,NH,DH) storage; di,df views of (B,S,NH) storage
-        dq3, dk3, dv3 = (t.transpose(1, 2).reshape(B, S, D) for t in (dq, dk, dv))
-        dw_i, db_i, dw_f, db_f = gate_proj_bwd_raw(q3, k3, v3, w_i, w_f, NH, di.transpose(1, 2), df.transpose(1, 2),
-                                                   dq3, dk3, dv3, need_bias=has_bias)
-        return dq3, dk3, dv3, dw_i, db_i, dw_f, db_f, None, None, None, None, None
+        grads = fused_cell_bwd_raw(*ctx.saved_tensors, dh, *ctx.cfg)
+        return grads + (None,) * 5
 
 
 def fused_cell(q3: torch.Tensor, k3: torch.Tensor, v3: torch.Tensor, w_i: torch.Tensor, b_i: Optional[torch.Tensor],
@@ -470,13 +521,19 @@ def fused_cell(q3: torch.Tensor, k3: torch.Tensor, v3: torch.Tensor, w_i: torch.
         kernel_dtype = torch.float32 if in_dtype == torch.float32 else torch.bfloat16
     if kernel_dtype not in _DT:
         raise ValueError(f"kernel_dtype must be float32 or bfloat16, got {kernel_dtype}")
-    q3, k3, v3 = (t.to(kernel_dtype) for t in (q3, k3, v3))
-    q3, k3, v3 = (t if _rows_ok(t) else t.contiguous() for t in (q3, k3, v3))
-    if q3.stride(1) != k3.stride(1) or q3.stride(1) != v3.stride(1):
-        q3, k3, v3 = q3.contiguous(), k3.contiguous(), v3.contiguous()
+    traced = _use_custom_ops()
+    # (a traced call cannot see addresses: the op copies a misaligned operand)
+    q3, k3, v3 = _cell_rows(*(t.to(kernel_dtype) for t in (q3, k3, v3)), rows_ok=_rows_layout_ok if traced else None)
     f32 = lambda t: None if t is None else t.to(torch.float32).contiguous()
-    h = _FusedCellFn.apply(q3, k3, v3, f32(w_i), f32(b_i), f32(w_f), f32(b_f), int(num_heads), float(eps),
-                           int(chunk_size), bool(reverse), gate_mode_of(input_gate))
+    args = (q3, k3, v3, f32(w_i), f32(b_i), f32(w_f), f32(b_f), int(num_heads), float(eps), int(chunk_size), bool(reverse),
+            gate_mode_of(input_gate))
+    if traced:
+        save_rows = torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in args[:7])
+        B, S, D = q3.shape
+        nbytes = _states_numel(B, num_heads, S, D // num_heads, D // num_heads, kernel_dtype)
+        h = _fused_cell_fwd_op(*args, save_rows, nbytes)[0]
+    else:
+        h = _FusedCellFn.apply(*args)
     return h.to(in_dtype)
 
 
@@ -489,11 +546,16 @@ def glue_supported(h: torch.Tensor, c: torch.Tensor, z: torch.Tensor) -> bool:
         return False
     B, NH, S, DH = h.shape
     D = NH * DH
-    if not _lib.load().mlstm_b200_glue_supported(D, NH):   # the C-side shape gate (D / 256 in {1, 2, 4, 8}, DH | 256)
+    if not _glue_lib_ok(int(D), int(NH)):   # the C-side shape gate (D / 256 in {1, 2, 4, 8}, DH | 256)
         return False
-    if h.stride() != (S * D, DH, D, 1) or h.data_ptr() % 16:
+    if h.stride() != (S * D, DH, D, 1) or not _aligned(h):
         return False
-    return all(t.dtype == h.dtype and t.shape == (B, S, D) and _rows_ok(t) for t in (c, z))
+    return all(t.dtype == h.dtype and t.shape == (B, S, D) and _rows_layout_ok(t) and _aligned(t) for t in (c, z))
+
+
+@torch.compiler.assume_constant_result
+def _glue_lib_ok(D: int, NH: int) -> bool:
+    return bool(_lib.load().mlstm_b200_glue_supported(int(D), int(NH)))
 
 
 def _glue_params(h, c, z, w, b, skip, eps) -> GlueParams:
@@ -510,53 +572,63 @@ def _glue_params(h, c, z, w, b, skip, eps) -> GlueParams:
     return g
 
 
+def layer_tail_fwd_raw(h, c, z, w, b, skip, eps):
+    """One tail forward launch on operands ``glue_supported`` accepts: y (B,S,D) in h's dtype."""
+    lib = _lib.load()
+    B, NH, S, DH = h.shape
+    y = torch.empty((B, S, NH * DH), dtype=h.dtype, device=h.device)
+    g = _glue_params(h, c, z, w, b, skip, eps)
+    g.y, g.ld_y = y.data_ptr(), NH * DH
+    with torch.cuda.device(h.device):
+        rc = lib.mlstm_b200_glue_fwd(C.byref(g), _stream())
+    if rc:
+        _fail(rc, "layer tail forward")
+    return y
+
+
+def layer_tail_bwd_raw(h, c, z, w, b, skip, dy, eps):
+    """One tail backward launch: (dh, dc, dz, dw, db, dskip); dh in h's layout, dc, dz dense, dw, db, dskip fp32 (D)
+    or None where the forward had no such parameter."""
+    lib = _lib.load()
+    B, NH, S, DH = h.shape
+    D = NH * DH
+    dev = h.device
+    if dy.dtype != h.dtype:
+        dy = dy.to(h.dtype)
+    if not _rows_ok(dy):
+        dy = dy.contiguous()
+    dh = _empty_act(B, NH, S, DH, h.dtype, dev)
+    dc = torch.empty((B, S, D), dtype=h.dtype, device=dev)
+    dz = torch.empty((B, S, D), dtype=h.dtype, device=dev)
+    dw = torch.empty(D, dtype=torch.float32, device=dev) if w is not None else None
+    db = torch.empty(D, dtype=torch.float32, device=dev) if b is not None else None
+    dskip = torch.empty(D, dtype=torch.float32, device=dev) if skip is not None else None
+    g = _glue_params(h, c, z, w, b, skip, eps)
+    g.dy, g.ld_dy = dy.data_ptr(), dy.stride(1)
+    g.dh, g.ld_dh = dh.data_ptr(), D
+    g.dc, g.ld_dc = dc.data_ptr(), D
+    g.dz, g.ld_dz = dz.data_ptr(), D
+    g.dw, g.db, g.dskip = _ptr(dw), _ptr(db), _ptr(dskip)
+    need = lib.mlstm_b200_glue_workspace_bytes(C.byref(g))
+    ws = torch.empty(max(1, (need + 3) // 4), dtype=torch.float32, device=dev)
+    g.workspace, g.workspace_bytes = ws.data_ptr(), ws.numel() * 4
+    with torch.cuda.device(dev):
+        rc = lib.mlstm_b200_glue_bwd(C.byref(g), _stream())
+    if rc:
+        _fail(rc, "layer tail backward")
+    return dh, dc, dz, dw, db, dskip
+
+
 class _GlueFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, h, c, z, w, b, skip, eps):
-        lib = _lib.load()
-        B, NH, S, DH = h.shape
-        y = torch.empty((B, S, NH * DH), dtype=h.dtype, device=h.device)
-        g = _glue_params(h, c, z, w, b, skip, eps)
-        g.y, g.ld_y = y.data_ptr(), NH * DH
-        with torch.cuda.device(h.device):
-            rc = lib.mlstm_b200_glue_fwd(C.byref(g), _stream())
-        if rc:
-            _fail(rc, "layer tail forward")
         ctx.save_for_backward(h, c, z, w, b, skip)
         ctx.eps = eps
-        return y
+        return layer_tail_fwd_raw(h, c, z, w, b, skip, eps)
 
     @staticmethod
     def backward(ctx, dy):
-        lib = _lib.load()
-        h, c, z, w, b, skip = ctx.saved_tensors
-        B, NH, S, DH = h.shape
-        D = NH * DH
-        dev = h.device
-        if dy.dtype != h.dtype:
-            dy = dy.to(h.dtype)
-        if not _rows_ok(dy):
-            dy = dy.contiguous()
-        dh = _empty_act(B, NH, S, DH, h.dtype, dev)
-        dc = torch.empty((B, S, D), dtype=h.dtype, device=dev)
-        dz = torch.empty((B, S, D), dtype=h.dtype, device=dev)
-        dw = torch.empty(D, dtype=torch.float32, device=dev) if w is not None else None
-        db = torch.empty(D, dtype=torch.float32, device=dev) if b is not None else None
-        dskip = torch.empty(D, dtype=torch.float32, device=dev) if skip is not None else None
-        g = _glue_params(h, c, z, w, b, skip, ctx.eps)
-        g.dy, g.ld_dy = dy.data_ptr(), dy.stride(1)
-        g.dh, g.ld_dh = dh.data_ptr(), D
-        g.dc, g.ld_dc = dc.data_ptr(), D
-        g.dz, g.ld_dz = dz.data_ptr(), D
-        g.dw, g.db, g.dskip = _ptr(dw), _ptr(db), _ptr(dskip)
-        need = lib.mlstm_b200_glue_workspace_bytes(C.byref(g))
-        ws = torch.empty(max(1, (need + 3) // 4), dtype=torch.float32, device=dev)
-        g.workspace, g.workspace_bytes = ws.data_ptr(), ws.numel() * 4
-        with torch.cuda.device(dev):
-            rc = lib.mlstm_b200_glue_bwd(C.byref(g), _stream())
-        if rc:
-            _fail(rc, "layer tail backward")
-        return dh, dc, dz, dw, db, dskip, None
+        return layer_tail_bwd_raw(*ctx.saved_tensors, dy, ctx.eps) + (None,)
 
 
 def layer_tail(h: torch.Tensor, conv_act: torch.Tensor, z: torch.Tensor, norm_weight: Optional[torch.Tensor],
@@ -564,7 +636,10 @@ def layer_tail(h: torch.Tensor, conv_act: torch.Tensor, z: torch.Tensor, norm_we
     """``(LN_head(h) * (1 + w) + b + skip * conv_act) * silu(z)`` -> (B,S,D).  ``h`` is the raw cell output
     (B,NH,S,DH); check ``glue_supported`` first."""
     f32 = lambda t: None if t is None else t.to(torch.float32).contiguous()
-    return _GlueFn.apply(h, conv_act, z, f32(norm_weight), f32(norm_bias), f32(skip), float(eps))
+    args = (h, conv_act, z, f32(norm_weight), f32(norm_bias), f32(skip), float(eps))
+    if _use_custom_ops():
+        return _layer_tail_fwd_op(*args)
+    return _GlueFn.apply(*args)
 
 
 # ---------------------------------------------------------------------------------------------------------------
@@ -575,9 +650,14 @@ def qkv_supported(x: torch.Tensor, D: int, NH: int, gh: int, gw: int) -> bool:
     """x: (B,S,D) rows of proj_up's output (a column slice is fine), bf16 or fp16 on CUDA."""
     if not x.is_cuda or x.dtype not in (torch.bfloat16, torch.float16) or x.dim() != 3 or x.shape[1] != gh * gw:
         return False
-    if x.stride(2) != 1 or x.stride(0) != x.shape[1] * x.stride(1) or x.data_ptr() % 16:
+    if x.stride(2) != 1 or x.stride(0) != x.shape[1] * x.stride(1) or not _aligned(x):
         return False
-    return bool(_lib.load().mlstm_b200_qkv_supported(int(D), int(NH), int(gh), int(gw), int(x.stride(1))))
+    return _qkv_lib_ok(int(D), int(NH), int(gh), int(gw), int(x.stride(1)))
+
+
+@torch.compiler.assume_constant_result
+def _qkv_lib_ok(D: int, NH: int, gh: int, gw: int, ld: int) -> bool:
+    return bool(_lib.load().mlstm_b200_qkv_supported(D, NH, gh, gw, ld))
 
 
 def qkv_reference(x, conv_w, conv_b, wq, bq, wk, bk, wv, bv, gh, gw, rotate=False):
@@ -756,34 +836,49 @@ def qkv_backward(x, c, conv_w, conv_b, wq, wk, wv, has_bias, dc, dq, dk, dv, gh,
     return (dx, dwc, dbc, dwq, sums[0], dwk, sums[1], dwv, sums[2])
 
 
+def qkv_fwd_raw(x, conv_w, conv_b, wq, bq, wk, bk, wv, bv, gh, gw, rotate, need_sp):
+    """One producer forward launch on an ``x`` that ``qkv_supported`` accepts: (c, q, k, v, sp), each (B,S,D) bf16;
+    sp = silu'(conv(x)), which the conv's backward kernel reads, only when ``need_sp`` (else None)."""
+    lib = _lib.load()
+    B, S, D = x.shape
+    NH = wq.shape[0]
+    dev = x.device
+    f32 = lambda t: None if t is None else t.detach().to(torch.float32).contiguous()
+    cw, cb, fbq, fbk, fbv = f32(conv_w), f32(conv_b), f32(bq), f32(bk), f32(bv)
+    kq, kk = wq.detach().to(torch.bfloat16).contiguous(), wk.detach().to(torch.bfloat16).contiguous()
+    kv = wv.detach().to(x.dtype).contiguous()
+    c, q, k, v = (torch.empty((B, S, D), dtype=torch.bfloat16, device=dev) for _ in range(4))
+    sp = torch.empty((B, S, D), dtype=torch.bfloat16, device=dev) if need_sp else None
+    g = QkvParams()
+    g.abi_version = _lib.ABI_VERSION
+    g.B, g.GH, g.GW, g.D, g.NH = B, gh, gw, D, NH
+    g.rotate, g.x_dtype = int(bool(rotate)), int(x.dtype == torch.float16)
+    g.x, g.ld_x = x.data_ptr(), x.stride(1)
+    g.conv_w, g.conv_b = cw.data_ptr(), _ptr(cb)
+    g.wq, g.wk, g.wv = kq.data_ptr(), kk.data_ptr(), kv.data_ptr()
+    g.bq, g.bk, g.bv = _ptr(fbq), _ptr(fbk), _ptr(fbv)
+    g.c, g.q, g.k, g.v = c.data_ptr(), q.data_ptr(), k.data_ptr(), v.data_ptr()
+    g.sp = _ptr(sp)
+    with torch.cuda.device(dev):
+        rc = lib.mlstm_b200_qkv_fwd(C.byref(g), _stream())
+    if rc:
+        _fail(rc, "qkv producer forward")
+    return c, q, k, v, sp
+
+
+def _qkv_grads(x, c, conv_w, conv_b, wq, wk, wv, sp, dc, dq, dk, dv, gh, gw, rotate, has_bias):
+    """``qkv_backward`` with each gradient in its input's dtype (the projections' bias gradients stay fp32)."""
+    g = qkv_backward(x, c, conv_w, conv_b, wq, wk, wv, has_bias, dc, dq, dk, dv, gh, gw, rotate, sp=sp)
+    dx, dwc, dbc, dwq, dbq, dwk, dbk, dwv, dbv = g
+    cast = lambda t, like: None if (t is None or like is None) else t.to(like.dtype)
+    return dx.to(x.dtype), cast(dwc, conv_w), cast(dbc, conv_b), cast(dwq, wq), dbq, cast(dwk, wk), dbk, cast(dwv, wv), dbv
+
+
 class _QkvFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, conv_w, conv_b, wq, bq, wk, bk, wv, bv, gh, gw, rotate):
-        lib = _lib.load()
-        B, S, D = x.shape
-        NH = wq.shape[0]
-        dev = x.device
-        f32 = lambda t: None if t is None else t.detach().to(torch.float32).contiguous()
-        cw, cb, fbq, fbk, fbv = f32(conv_w), f32(conv_b), f32(bq), f32(bk), f32(bv)
-        kq, kk = wq.detach().to(torch.bfloat16).contiguous(), wk.detach().to(torch.bfloat16).contiguous()
-        kv = wv.detach().to(x.dtype).contiguous()
-        c, q, k, v = (torch.empty((B, S, D), dtype=torch.bfloat16, device=dev) for _ in range(4))
         # silu'(conv(x)) for the conv's backward kernel: only when a backward can follow
-        sp = torch.empty((B, S, D), dtype=torch.bfloat16, device=dev) if any(ctx.needs_input_grad[:9]) else None
-        g = QkvParams()
-        g.abi_version = _lib.ABI_VERSION
-        g.B, g.GH, g.GW, g.D, g.NH = B, gh, gw, D, NH
-        g.rotate, g.x_dtype = int(bool(rotate)), int(x.dtype == torch.float16)
-        g.x, g.ld_x = x.data_ptr(), x.stride(1)
-        g.conv_w, g.conv_b = cw.data_ptr(), _ptr(cb)
-        g.wq, g.wk, g.wv = kq.data_ptr(), kk.data_ptr(), kv.data_ptr()
-        g.bq, g.bk, g.bv = _ptr(fbq), _ptr(fbk), _ptr(fbv)
-        g.c, g.q, g.k, g.v = c.data_ptr(), q.data_ptr(), k.data_ptr(), v.data_ptr()
-        g.sp = _ptr(sp)
-        with torch.cuda.device(dev):
-            rc = lib.mlstm_b200_qkv_fwd(C.byref(g), _stream())
-        if rc:
-            _fail(rc, "qkv producer forward")
+        c, q, k, v, sp = qkv_fwd_raw(x, conv_w, conv_b, wq, bq, wk, bk, wv, bv, gh, gw, rotate, any(ctx.needs_input_grad[:9]))
         ctx.save_for_backward(x, c, conv_w, conv_b, wq, wk, wv, sp)
         ctx.meta = (gh, gw, bool(rotate), (bq is not None, bk is not None, bv is not None))
         return c, q, k, v
@@ -793,17 +888,17 @@ class _QkvFn(torch.autograd.Function):
         x, c, conv_w, conv_b, wq, wk, wv, sp = ctx.saved_tensors
         gh, gw, rotate, has_bias = ctx.meta
         z = lambda t: torch.zeros_like(c) if t is None else t
-        g = qkv_backward(x, c, conv_w, conv_b, wq, wk, wv, has_bias, dc, z(dq), z(dk), z(dv), gh, gw, rotate, sp=sp)
-        dx, dwc, dbc, dwq, dbq, dwk, dbk, dwv, dbv = g
-        cast = lambda t, like: None if (t is None or like is None) else t.to(like.dtype)
-        return (dx.to(x.dtype), cast(dwc, conv_w), cast(dbc, conv_b), cast(dwq, wq), dbq, cast(dwk, wk), dbk, cast(dwv, wv), dbv,
-                None, None, None)
+        return _qkv_grads(x, c, conv_w, conv_b, wq, wk, wv, sp, dc, z(dq), z(dk), z(dv), gh, gw, rotate, has_bias) + (None,) * 3
 
 
 def qkv_producer(x, conv_w, conv_b, wq, bq, wk, bk, wv, bv, gh: int, gw: int, rotate: bool = False):
     """(c, q, k, v) = (silu(conv(x)), c Wq^T + bq, c Wk^T + bk, x Wv^T + bv), all (B,S,D) bf16, from one kernel
     (csrc/mlstm_qkv.cu).  Check ``qkv_supported`` first.  Backward: ``qkv_backward`` (cuBLAS / cuDNN through PyTorch)."""
-    return _QkvFn.apply(x, conv_w, conv_b, wq, bq, wk, bk, wv, bv, int(gh), int(gw), bool(rotate))
+    args = (x, conv_w, conv_b, wq, bq, wk, bk, wv, bv, int(gh), int(gw), bool(rotate))
+    if _use_custom_ops():
+        need_sp = torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in args[:9])
+        return _qkv_fwd_op(*args, need_sp)[:4]
+    return _QkvFn.apply(*args)
 
 
 class MLSTMPlan:
@@ -853,3 +948,207 @@ class MLSTMPlan:
         if rc:
             _fail(rc, "backward")
         return self.dq, self.dk, self.dv, self.di, self.df
+
+
+# ---------------------------------------------------------------------------------------------------------------
+# torch.library registration of the layer kernels: ``xlstm_yolo_b200::fused_cell_fwd`` / ``::fused_cell_bwd``,
+# ``::qkv_fwd`` / ``::qkv_bwd`` and ``::layer_tail_fwd`` / ``::layer_tail_bwd`` call the launchers above, so a compiled
+# model runs the same kernels as an eager one.  The fakes give the real layouts (Inductor checks the sizes and strides of
+# what an op returns).  An absent optional output is an empty tensor, mapped to None in the autograd formulas.  The
+# caller sizes the chunk-state buffer (``_states_numel``), so that a dynamic batch needs no data-dependent output size.
+# ---------------------------------------------------------------------------------------------------------------
+def _use_custom_ops() -> bool:
+    """torch.compile traces the custom ops; eager mode calls the autograd.Functions: same launches, less host time.
+    Measured on a B200 (1000 W limit, tests/gpu_tools/compile_bench.py), eager ViLBlockPair forward + backward, twelve
+    layer-op calls per step: 3.21 ms through the autograd.Functions vs 4.14 ms through the custom ops at dim 128, B 32,
+    400 tokens (about 80 us more per call), 3.68 vs 4.19-4.41 ms at dim 256, B 32, 1600 tokens."""
+    return torch.compiler.is_compiling()
+
+
+def _none_to_empty(t: Optional[torch.Tensor], like: torch.Tensor, dtype=torch.float32) -> torch.Tensor:
+    return torch.empty(0, dtype=dtype, device=like.device) if t is None else t
+
+
+def _tail_h(h: torch.Tensor) -> torch.Tensor:
+    """h as the tail kernel reads it: a 16-byte aligned (B,NH,S,DH) view of (B,S,NH,DH) storage, else a copy into one."""
+    B, NH, S, DH = h.shape
+    if h.stride() == (S * NH * DH, DH, NH * DH, 1) and h.data_ptr() % 16 == 0:
+        return h
+    out = _empty_act(B, NH, S, DH, h.dtype, h.device)
+    out.copy_(h)
+    return out
+
+
+def _dense_rows(t: torch.Tensor) -> torch.Tensor:
+    return t if _rows_ok(t) else t.contiguous()
+
+
+@torch.library.custom_op("xlstm_yolo_b200::fused_cell_fwd", mutates_args=(), device_types="cuda")
+def _fused_cell_fwd_op(q3: torch.Tensor, k3: torch.Tensor, v3: torch.Tensor, w_i: torch.Tensor, b_i: Optional[torch.Tensor],
+                       w_f: torch.Tensor, b_f: Optional[torch.Tensor], num_heads: int, eps: float, chunk_size: int, reverse: bool,
+                       gate_mode: int, save_rows: bool,
+                       states_bytes: int) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
+    q3, k3, v3 = _cell_rows(q3, k3, v3)
+    h, i3, f3, n_row, m_row, states = fused_cell_fwd_raw(q3, k3, v3, w_i, b_i, w_f, b_f, num_heads, eps, chunk_size, reverse,
+                                                         gate_mode, save_rows, states_bytes)
+    return h, i3, f3, _none_to_empty(n_row, h), _none_to_empty(m_row, h), _none_to_empty(states, h, torch.uint8)
+
+
+@_fused_cell_fwd_op.register_fake
+def _(q3, k3, v3, w_i, b_i, w_f, b_f, num_heads, eps, chunk_size, reverse, gate_mode, save_rows, states_bytes):
+    B, S, D = q3.shape
+    NH, DH, dev = num_heads, D // num_heads, q3.device
+    h = torch.empty((B, S, NH, DH), dtype=q3.dtype, device=dev).transpose(1, 2)
+    i3, f3 = (torch.empty((B, S, NH), dtype=torch.float32, device=dev) for _ in range(2))
+    rows = (lambda: torch.empty((B, NH, S), dtype=torch.float32, device=dev)) if save_rows else \
+        (lambda: torch.empty(0, dtype=torch.float32, device=dev))
+    states = torch.empty(states_bytes, dtype=torch.uint8, device=dev)
+    return h, i3, f3, rows(), rows(), states
+
+
+@torch.library.custom_op("xlstm_yolo_b200::fused_cell_bwd", mutates_args=(), device_types="cuda")
+def _fused_cell_bwd_op(q3: torch.Tensor, k3: torch.Tensor, v3: torch.Tensor, w_i: torch.Tensor, w_f: torch.Tensor,
+                       i3: torch.Tensor, f3: torch.Tensor, h: torch.Tensor, n_row: torch.Tensor, m_row: torch.Tensor,
+                       states: torch.Tensor, dh: torch.Tensor, num_heads: int, eps: float, chunk_size: int, reverse: bool,
+                       gate_mode: int, has_bias: bool) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor,
+                                                                torch.Tensor, torch.Tensor, torch.Tensor]:
+    q3, k3, v3 = _cell_rows(q3, k3, v3)
+    dq3, dk3, dv3, dw_i, db_i, dw_f, db_f = fused_cell_bwd_raw(
+        q3, k3, v3, w_i, w_f, i3, f3, _prep_act(h), n_row, m_row, states if states.numel() else None, dh, num_heads, eps,
+        chunk_size, reverse, gate_mode, has_bias)
+    return dq3, dk3, dv3, dw_i, _none_to_empty(db_i, h), dw_f, _none_to_empty(db_f, h)
+
+
+@_fused_cell_bwd_op.register_fake
+def _(q3, k3, v3, w_i, w_f, i3, f3, h, n_row, m_row, states, dh, num_heads, eps, chunk_size, reverse, gate_mode, has_bias):
+    B, S, D = q3.shape
+    d3 = lambda: torch.empty((B, S, D), dtype=q3.dtype, device=q3.device)
+    db = lambda: torch.empty(num_heads if has_bias else 0, dtype=torch.float32, device=q3.device)
+    return d3(), d3(), d3(), torch.empty_like(w_i), db(), torch.empty_like(w_f), db()
+
+
+def _fused_cell_setup_context(ctx, inputs, output):
+    q3, k3, v3, w_i, b_i, w_f, b_f, num_heads, eps, chunk_size, reverse, gate_mode, save_rows, states_bytes = inputs
+    h, i3, f3, n_row, m_row, states = output
+    ctx.save_for_backward(q3, k3, v3, w_i, w_f, i3, f3, h, n_row, m_row, states)
+    ctx.cfg = (num_heads, eps, chunk_size, reverse, gate_mode, b_i is not None)
+    ctx.set_materialize_grads(False)
+
+
+def _fused_cell_backward(ctx, dh, *_unused):
+    saved = ctx.saved_tensors
+    if dh is None:
+        dh = torch.zeros_like(saved[7])
+    dq3, dk3, dv3, dw_i, db_i, dw_f, db_f = _fused_cell_bwd_op(*saved, dh, *ctx.cfg)
+    has_bias = ctx.cfg[-1]
+    return (dq3, dk3, dv3, dw_i, db_i if has_bias else None, dw_f, db_f if has_bias else None) + (None,) * 7
+
+
+_fused_cell_fwd_op.register_autograd(_fused_cell_backward, setup_context=_fused_cell_setup_context)
+
+
+@torch.library.custom_op("xlstm_yolo_b200::qkv_fwd", mutates_args=(), device_types="cuda")
+def _qkv_fwd_op(x: torch.Tensor, conv_w: torch.Tensor, conv_b: Optional[torch.Tensor], wq: torch.Tensor, bq: Optional[torch.Tensor],
+                wk: torch.Tensor, bk: Optional[torch.Tensor], wv: torch.Tensor, bv: Optional[torch.Tensor], gh: int, gw: int,
+                rotate: bool, need_sp: bool) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
+    c, q, k, v, sp = qkv_fwd_raw(_dense_rows(x), conv_w, conv_b, wq, bq, wk, bk, wv, bv, gh, gw, rotate, need_sp)
+    return c, q, k, v, _none_to_empty(sp, x, torch.bfloat16)
+
+
+@_qkv_fwd_op.register_fake
+def _(x, conv_w, conv_b, wq, bq, wk, bk, wv, bv, gh, gw, rotate, need_sp):
+    act = lambda: torch.empty(x.shape, dtype=torch.bfloat16, device=x.device)
+    return act(), act(), act(), act(), act() if need_sp else torch.empty(0, dtype=torch.bfloat16, device=x.device)
+
+
+@torch.library.custom_op("xlstm_yolo_b200::qkv_bwd", mutates_args=(), device_types="cuda")
+def _qkv_bwd_op(x: torch.Tensor, c: torch.Tensor, conv_w: torch.Tensor, conv_b: Optional[torch.Tensor], wq: torch.Tensor,
+                wk: torch.Tensor, wv: torch.Tensor, sp: torch.Tensor, dc: Optional[torch.Tensor], dq: torch.Tensor, dk: torch.Tensor,
+                dv: torch.Tensor, gh: int, gw: int, rotate: bool, has_bq: bool, has_bk: bool,
+                has_bv: bool) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor,
+                                       torch.Tensor, torch.Tensor, torch.Tensor]:
+    grads = _qkv_grads(_dense_rows(x), c, conv_w, conv_b, wq, wk, wv, sp if sp.numel() else None, dc, dq, dk, dv, gh, gw,
+                       rotate, (has_bq, has_bk, has_bv))
+    # outputs own their storage: the projections' bias gradients may be rows of one (3, D) buffer
+    return tuple(_none_to_empty(t, x) if t is None else t.clone() if j in (4, 6, 8) else t.contiguous()
+                 for j, t in enumerate(grads))
+
+
+@_qkv_bwd_op.register_fake
+def _(x, c, conv_w, conv_b, wq, wk, wv, sp, dc, dq, dk, dv, gh, gw, rotate, has_bq, has_bk, has_bv):
+    D, dev = x.shape[2], x.device
+    bias = lambda on: torch.empty(D if on else 0, dtype=torch.float32, device=dev)
+    return (torch.empty(x.shape, dtype=x.dtype, device=dev), torch.empty(conv_w.shape, dtype=conv_w.dtype, device=dev),
+            torch.empty(0, dtype=torch.float32, device=dev) if conv_b is None else torch.empty(D, dtype=conv_b.dtype, device=dev),
+            torch.empty(wq.shape, dtype=wq.dtype, device=dev), bias(has_bq), torch.empty(wk.shape, dtype=wk.dtype, device=dev),
+            bias(has_bk), torch.empty(wv.shape, dtype=wv.dtype, device=dev), bias(has_bv))
+
+
+def _qkv_setup_context(ctx, inputs, output):
+    x, conv_w, conv_b, wq, bq, wk, bk, wv, bv, gh, gw, rotate, need_sp = inputs
+    c, q, k, v, sp = output
+    ctx.save_for_backward(x, c, conv_w, conv_b, wq, wk, wv, sp)
+    ctx.meta = (gh, gw, rotate, bq is not None, bk is not None, bv is not None)
+    ctx.set_materialize_grads(False)
+
+
+def _qkv_backward(ctx, dc, dq, dk, dv, _dsp):
+    x, c, conv_w, conv_b, wq, wk, wv, sp = ctx.saved_tensors
+    z = lambda t: torch.zeros_like(c) if t is None else t
+    g = _qkv_bwd_op(x, c, conv_w, conv_b, wq, wk, wv, sp, dc, z(dq), z(dk), z(dv), *ctx.meta)
+    has_b = (conv_b is not None,) + ctx.meta[3:]
+    dx, dwc, dbc, dwq, dbq, dwk, dbk, dwv, dbv = g
+    pick = lambda t, on: t if on else None
+    return (dx, dwc, pick(dbc, has_b[0]), dwq, pick(dbq, has_b[1]), dwk, pick(dbk, has_b[2]), dwv, pick(dbv, has_b[3]),
+            None, None, None, None)
+
+
+_qkv_fwd_op.register_autograd(_qkv_backward, setup_context=_qkv_setup_context)
+
+
+@torch.library.custom_op("xlstm_yolo_b200::layer_tail_fwd", mutates_args=(), device_types="cuda")
+def _layer_tail_fwd_op(h: torch.Tensor, c: torch.Tensor, z: torch.Tensor, w: Optional[torch.Tensor], b: Optional[torch.Tensor],
+                       skip: Optional[torch.Tensor], eps: float) -> torch.Tensor:
+    return layer_tail_fwd_raw(_tail_h(h), _dense_rows(c), _dense_rows(z), w, b, skip, eps)
+
+
+@_layer_tail_fwd_op.register_fake
+def _(h, c, z, w, b, skip, eps):
+    B, NH, S, DH = h.shape
+    return torch.empty((B, S, NH * DH), dtype=h.dtype, device=h.device)
+
+
+@torch.library.custom_op("xlstm_yolo_b200::layer_tail_bwd", mutates_args=(), device_types="cuda")
+def _layer_tail_bwd_op(h: torch.Tensor, c: torch.Tensor, z: torch.Tensor, w: Optional[torch.Tensor], b: Optional[torch.Tensor],
+                       skip: Optional[torch.Tensor], dy: torch.Tensor,
+                       eps: float) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
+    dh, dc, dz, dw, db, dskip = layer_tail_bwd_raw(_tail_h(h), _dense_rows(c), _dense_rows(z), w, b, skip, dy, eps)
+    return dh, dc, dz, _none_to_empty(dw, h), _none_to_empty(db, h), _none_to_empty(dskip, h)
+
+
+@_layer_tail_bwd_op.register_fake
+def _(h, c, z, w, b, skip, dy, eps):
+    B, NH, S, DH = h.shape
+    D, dev = NH * DH, h.device
+    d3 = lambda: torch.empty((B, S, D), dtype=h.dtype, device=dev)
+    vec = lambda t: torch.empty(0 if t is None else D, dtype=torch.float32, device=dev)
+    return _empty_act(B, NH, S, DH, h.dtype, dev), d3(), d3(), vec(w), vec(b), vec(skip)
+
+
+def _layer_tail_setup_context(ctx, inputs, output):
+    h, c, z, w, b, skip, eps = inputs
+    ctx.save_for_backward(h, c, z, w, b, skip)
+    ctx.eps = eps
+    ctx.set_materialize_grads(False)
+
+
+def _layer_tail_backward(ctx, dy):
+    h, c, z, w, b, skip = ctx.saved_tensors
+    if dy is None:
+        return (None,) * 7
+    dh, dc, dz, dw, db, dskip = _layer_tail_bwd_op(h, c, z, w, b, skip, dy, ctx.eps)
+    pick = lambda t, like: None if like is None else t
+    return dh, dc, dz, pick(dw, w), pick(db, b), pick(dskip, skip), None
+
+
+_layer_tail_fwd_op.register_autograd(_layer_tail_backward, setup_context=_layer_tail_setup_context)

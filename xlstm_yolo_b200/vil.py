@@ -232,7 +232,7 @@ class ViLLayer(nn.Module):
         x_mlstm, z = self.proj_up(y).chunk(2, dim=-1)
         cell = self.mlstm_cell
         conv_act = None
-        if (x.is_cuda and getattr(self, "fused_producer", True) and not torch.compiler.is_compiling()
+        if (x.is_cuda and getattr(self, "fused_producer", True)
                 and self.conv.kernel_size == (3, 3) and self.conv.padding == (1, 1) and self.conv.stride == (1, 1)
                 and self.conv.dilation == (1, 1) and self.conv.groups == self.conv.in_channels == self.conv.out_channels):
             # conv + SiLU + the three block-diagonal projections as one kernel (vision_lstm2.py:482-491 are four
@@ -248,7 +248,7 @@ class ViLLayer(nn.Module):
             conv_act = F.silu(self.conv(x_mlstm, rotate=anti))
             q, k, v = self.q_proj(conv_act), self.k_proj(conv_act), self.v_proj(x_mlstm)
         y = None
-        if x.is_cuda and getattr(self, "fused_tail", True) and not cell.raw_output and not torch.compiler.is_compiling():
+        if x.is_cuda and getattr(self, "fused_tail", True) and not cell.raw_output:
             # out-norm + skip + SiLU(z) gate as one streaming kernel over the raw cell output
             # (vision_lstm2.py:950, :498-499 are four separate (B,S,inner) round trips).  Direction and output
             # form are call arguments: no module state is touched, so the forward is re-entrant.
