@@ -52,7 +52,7 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--mode", default="train", choices=["train", "infer"])
-    ap.add_argument("--scale", default="s", choices=["n", "s", "m"])
+    ap.add_argument("--scale", default="s", choices=["n", "s", "m", "l", "x"])
     ap.add_argument("--batch", type=int, default=64, help="GLOBAL batch (train: split over the ranks); per GPU for --mode infer")
     ap.add_argument("--imgsz", type=int, default=640)
     ap.add_argument("--device", default="cuda")

@@ -44,7 +44,9 @@
 extern "C" {
 #endif
 
-#define MLSTM_B200_ABI_VERSION 5
+/* ABI 6: mlstm_b200_gates_fwd may need a workspace (mlstm_b200_gates_fwd_workspace_bytes); callers built for ABI 5 passed
+ * none, so they are refused by the version check rather than failing at the shapes that need one. */
+#define MLSTM_B200_ABI_VERSION 6
 
 typedef enum mlstm_status {
   MLSTM_OK = 0,
@@ -154,7 +156,8 @@ typedef struct mlstm_gate_proj_params {
                                            cell's gradients are dense even when q,k,v are column slices) */
   float *dw_i, *dw_f;                   /* backward outputs (NH, 3*D), overwritten */
   float *db_i, *db_f;                   /* backward outputs (NH), overwritten; NULL allowed */
-  void* workspace;                      /* >= mlstm_b200_gates_workspace_bytes() (backward only) */
+  void* workspace;                      /* forward (ABI 6): >= mlstm_b200_gates_fwd_workspace_bytes(), 16-byte aligned,
+                                           may be NULL when that is 0; backward: >= mlstm_b200_gates_workspace_bytes() */
   size_t workspace_bytes;
 } mlstm_gate_proj_params;
 
@@ -162,6 +165,11 @@ typedef struct mlstm_gate_proj_params {
  * the 8 x 3D fp32 weight tile fits in shared memory (D <= 2133). */
 int mlstm_b200_gates_supported(int D, int64_t ld);
 size_t mlstm_b200_gates_workspace_bytes(const mlstm_gate_proj_params* p);
+/* Forward scratch (ABI 6): the bf16 hi / mid / lo split of the weights that the tensor-core forward (bf16 q, k, v with
+ * 16-byte aligned rows, D % 64 == 0, 2 * NH <= 32) streams next to q, k, v when the split does not fit in shared memory
+ * (3 * D / 64 slices of NR x 128 bytes above ~107 KB).  0 for shapes whose split stays in shared memory, for shapes the
+ * SIMT kernel takes and for shapes the forward refuses. */
+size_t mlstm_b200_gates_fwd_workspace_bytes(const mlstm_gate_proj_params* p);
 int mlstm_b200_gates_fwd(const mlstm_gate_proj_params* p, void* cuda_stream);
 int mlstm_b200_gates_bwd(const mlstm_gate_proj_params* p, void* cuda_stream);
 
@@ -194,8 +202,9 @@ typedef struct mlstm_glue_params {
   size_t workspace_bytes;
 } mlstm_glue_params;
 
-/* 1 when the fused tail handles (D, NH): D % 256 == 0 with D / 256 in {1, 2, 4, 8}, DH = D / NH a multiple of 8
- * dividing 256. */
+/* 1 when the fused tail handles (D, NH): D % 256 == 0 with D <= 2048, DH = D / NH a multiple of 8 dividing 256.
+ * A CTA runs (8 / nseg) * nseg warps for nseg = D / 256 (whole rows of 256-column warp segments), so the backward's
+ * per-CTA partials, and mlstm_b200_glue_workspace_bytes(), follow that CTA size. */
 int mlstm_b200_glue_supported(int D, int NH);
 size_t mlstm_b200_glue_workspace_bytes(const mlstm_glue_params* p);
 int mlstm_b200_glue_fwd(const mlstm_glue_params* p, void* cuda_stream);

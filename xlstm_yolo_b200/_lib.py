@@ -13,7 +13,7 @@ _PKG = os.path.dirname(os.path.abspath(__file__))
 # MLSTM_B200_LIB: developer override for A/B builds (build.build_variant); the product path is the in-tree library
 LIB_PATH = os.environ.get("MLSTM_B200_LIB") or os.path.join(_PKG, "lib", "libmlstm_b200.so")
 
-ABI_VERSION = 5
+ABI_VERSION = 6
 MLSTM_F32, MLSTM_BF16 = 0, 1
 
 STATUS = {0: "OK", -1: "INVALID_ARG", -2: "UNSUPPORTED", -3: "WORKSPACE", -4: "CUDA", -5: "NO_DEVICE"}
@@ -37,6 +37,7 @@ EXPORTS = (
     "mlstm_b200_colsum",
     "mlstm_b200_gates_supported",
     "mlstm_b200_gates_workspace_bytes",
+    "mlstm_b200_gates_fwd_workspace_bytes",
     "mlstm_b200_gates_fwd",
     "mlstm_b200_gates_bwd",
     "mlstm_b200_glue_supported",
@@ -208,6 +209,8 @@ def load() -> C.CDLL:
         lib.mlstm_b200_glue_supported.argtypes = [C.c_int, C.c_int]
         lib.mlstm_b200_gates_workspace_bytes.restype = C.c_size_t
         lib.mlstm_b200_gates_workspace_bytes.argtypes = [C.POINTER(GateProjParams)]
+        lib.mlstm_b200_gates_fwd_workspace_bytes.restype = C.c_size_t
+        lib.mlstm_b200_gates_fwd_workspace_bytes.argtypes = [C.POINTER(GateProjParams)]
         lib.mlstm_b200_gates_fwd.restype = C.c_int
         lib.mlstm_b200_gates_fwd.argtypes = [C.POINTER(GateProjParams), C.c_void_p]
         lib.mlstm_b200_gates_bwd.restype = C.c_int

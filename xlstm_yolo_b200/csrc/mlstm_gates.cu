@@ -15,6 +15,7 @@
 
 namespace mlstm {
 bool gates_tc_ok(const mlstm_gate_proj_params& p);                     // mlstm_gates_tc.cu
+size_t gates_tc_workspace_bytes(const mlstm_gate_proj_params& p);
 int gates_fwd_tc(const mlstm_gate_proj_params& p, cudaStream_t st);
 namespace {
 
@@ -340,13 +341,25 @@ size_t mlstm_b200_gates_workspace_bytes(const mlstm_gate_proj_params* p) {
   return sizeof(float) * (size_t)bwd_ranges(*p) * (NO * C3 + NO);
 }
 
+size_t mlstm_b200_gates_fwd_workspace_bytes(const mlstm_gate_proj_params* p) {
+  if (!p || p->T <= 0 || p->D < 1 || p->NH < 1 || !mlstm_b200_gates_supported(p->D, p->ld) || !gates_tc_ok(*p)) return 0;
+  return gates_tc_workspace_bytes(*p);
+}
+
 int mlstm_b200_gates_fwd(const mlstm_gate_proj_params* p, void* cuda_stream) {
   clear_error();
   int rc = validate(p, false);
   if (rc || p->T == 0) return rc;
+  if (gates_tc_ok(*p)) {   // bf16, D % 64 == 0, <= 32 gate outputs: the tensor-core kernel (streamed weights need the workspace)
+    const size_t need = gates_tc_workspace_bytes(*p);
+    if (need && (!p->workspace || p->workspace_bytes < need || (uintptr_t)p->workspace % 16)) {
+      set_error("forward workspace too small or misaligned: need %zu bytes (16-byte aligned), got %zu", need, p->workspace_bytes);
+      return MLSTM_ERR_WORKSPACE;
+    }
+  }
   if ((rc = bind_device(p->q))) return rc;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(cuda_stream);
-  if (gates_tc_ok(*p)) return gates_fwd_tc(*p, st);   // bf16, D % 64 == 0, <= 16 gate outputs: the tensor-core streaming kernel
+  if (gates_tc_ok(*p)) return gates_fwd_tc(*p, st);
   const size_t smem = (size_t)OG * 3 * p->D * sizeof(float);
   const int tiles = (p->T + TT - 1) / TT, warps = FW_NT / 32;
   int grid = (tiles + warps - 1) / warps;

@@ -13,15 +13,23 @@
 // cell kernels write, seen as (T, D); every operand has its own row stride (z is a column slice of
 // proj_up's output).  A warp owns one 256-column segment of a token row (whole heads: DH divides 256),
 // a lane 8 adjacent columns (one 16-byte bf16 load); per-head statistics are xor-shuffle reductions over
-// the DH/8 lanes of the head.  HBM-bound row work: no shared-memory staging, no tensor cores.
+// the DH/8 lanes of the head.  A CTA is a whole number of rows: (8 / nseg) * nseg warps for nseg = D / 256
+// segments (8 warps at D = 256, 512, 1024, 2048; 6 at D = 768 and 1536; 5 at 1280; 7 at 1792), so warp w
+// of a CTA always owns segment w % nseg.  HBM-bound row work: no shared-memory staging, no tensor cores.
 #include "mlstm_common.cuh"
 
 namespace mlstm {
 namespace {
 
-constexpr int GL_NT = 256;                 // 8 warps
+constexpr int GL_NT = 256;                 // at most 8 warps
 constexpr int GL_EPL = 8;                  // elements per lane
 constexpr int GL_SEG = 32 * GL_EPL;        // columns per warp segment
+
+// warps per CTA: the most whole rows of D / GL_SEG segments that fit in GL_NT threads
+__host__ __device__ __forceinline__ int glue_warps(int D) {
+  const int nseg = D / GL_SEG;
+  return (GL_NT / 32 / nseg) * nseg;
+}
 
 template <typename T> struct Ld8;
 template <> struct Ld8<__nv_bfloat16> {
@@ -83,8 +91,8 @@ __device__ __forceinline__ void head_norm(const float* x, int lph, float inv_dh,
 
 template <typename T>
 __global__ void __launch_bounds__(GL_NT) glue_fwd_kernel(const mlstm_glue_params p) {
-  const int lane = threadIdx.x & 31;
-  const int gw = blockIdx.x * (GL_NT / 32) + (threadIdx.x >> 5), nw = gridDim.x * (GL_NT / 32);
+  const int lane = threadIdx.x & 31, wpc = blockDim.x >> 5;
+  const int gw = blockIdx.x * wpc + (threadIdx.x >> 5), nw = gridDim.x * wpc;
   const int nseg = p.D / GL_SEG, DH = p.D / p.NH, lph = DH / GL_EPL;
   const int seg = gw % nseg, col = seg * GL_SEG + lane * GL_EPL;
   const float inv_dh = 1.f / (float)DH;
@@ -123,8 +131,8 @@ __global__ void __launch_bounds__(GL_NT) glue_fwd_kernel(const mlstm_glue_params
 template <typename T>
 __global__ void __launch_bounds__(GL_NT, 2) glue_bwd_kernel(const mlstm_glue_params p, float* __restrict__ ws) {
   __shared__ float red[GL_NT / 32][3][GL_SEG];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int gw = blockIdx.x * (GL_NT / 32) + warp, nw = gridDim.x * (GL_NT / 32);
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, wpc = blockDim.x >> 5;
+  const int gw = blockIdx.x * wpc + warp, nw = gridDim.x * wpc;
   const int nseg = p.D / GL_SEG, DH = p.D / p.NH, lph = DH / GL_EPL;
   const int seg = gw % nseg, col = seg * GL_SEG + lane * GL_EPL;
   const float inv_dh = 1.f / (float)DH;
@@ -188,10 +196,10 @@ __global__ void __launch_bounds__(GL_NT, 2) glue_bwd_kernel(const mlstm_glue_par
     red[warp][2][lane * 8 + e] = as[e];
   }
   __syncthreads();
-  for (int i = threadIdx.x; i < 3 * p.D; i += GL_NT) {
+  for (int i = threadIdx.x; i < 3 * p.D; i += blockDim.x) {
     const int k = i / p.D, cd = i - k * p.D, sg = cd / GL_SEG, cc = cd - sg * GL_SEG;
     float acc = 0.f;
-    for (int w = sg; w < GL_NT / 32; w += nseg) acc += red[w][k][cc];   // warp w of a CTA owns segment w % nseg
+    for (int w = sg; w < wpc; w += nseg) acc += red[w][k][cc];   // warp w of a CTA owns segment w % nseg
     ws[((size_t)blockIdx.x * 3 + k) * p.D + cd] = acc;
   }
 }
@@ -207,8 +215,8 @@ __global__ void glue_reduce_kernel(const mlstm_glue_params p, const float* __res
 
 int glue_grid(const mlstm_glue_params& p) {
   const int nseg = p.D / GL_SEG;
-  const long long units = (long long)p.T * nseg;                 // (token, segment) work units, one per warp step
-  long long g = (units + (GL_NT / 32) * 4 - 1) / ((GL_NT / 32) * 4);   // >= 4 units per warp
+  const long long units = (long long)p.T * nseg, wpc = glue_warps(p.D);   // (token, segment) work units, one per warp step
+  long long g = (units + wpc * 4 - 1) / (wpc * 4);                  // >= 4 units per warp
   if (g > 2 * 148) g = 2 * 148;                                  // fixed cap: workspace size independent of the device
   return g < 1 ? 1 : (int)g;
 }
@@ -222,7 +230,7 @@ int validate(const mlstm_glue_params* p, bool bwd) {
   if (p->T < 0 || p->D < 1 || p->NH < 1 || p->D % p->NH) { set_error("bad sizes T=%d D=%d NH=%d", p->T, p->D, p->NH); return MLSTM_ERR_INVALID_ARG; }
   if (p->dtype != MLSTM_F32 && p->dtype != MLSTM_BF16) { set_error("unknown dtype %d", p->dtype); return MLSTM_ERR_UNSUPPORTED; }
   const int DH = p->D / p->NH;
-  if (p->D % GL_SEG || DH % GL_EPL || GL_SEG % DH || (GL_NT / 32) % (p->D / GL_SEG)) {
+  if (p->D % GL_SEG || p->D > GL_SEG * (GL_NT / 32) || DH % GL_EPL || GL_SEG % DH) {
     set_error("fused layer tail needs D a multiple of 256 (<= 2048) and DH in {8,...,256} dividing 256 (D=%d, DH=%d)", p->D, DH);
     return MLSTM_ERR_UNSUPPORTED;
   }
@@ -266,11 +274,11 @@ extern "C" {
 int mlstm_b200_glue_supported(int D, int NH) {
   if (D < 1 || NH < 1 || D % NH) return 0;
   const int DH = D / NH;
-  return !(D % GL_SEG || DH % GL_EPL || GL_SEG % DH || (GL_NT / 32) % (D / GL_SEG));
+  return !(D % GL_SEG || D > GL_SEG * (GL_NT / 32) || DH % GL_EPL || GL_SEG % DH);
 }
 
 size_t mlstm_b200_glue_workspace_bytes(const mlstm_glue_params* p) {
-  if (!p || p->T <= 0 || p->D < GL_SEG) return 0;
+  if (!p || p->T <= 0 || p->D < GL_SEG || p->D > GL_SEG * (GL_NT / 32)) return 0;
   return sizeof(float) * 3 * (size_t)p->D * glue_grid(*p);
 }
 
@@ -281,8 +289,8 @@ int mlstm_b200_glue_fwd(const mlstm_glue_params* p, void* cuda_stream) {
   if ((rc = bind_device(p->h))) return rc;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(cuda_stream);
   const int grid = glue_grid(*p);
-  if (p->dtype == MLSTM_BF16) glue_fwd_kernel<__nv_bfloat16><<<grid, GL_NT, 0, st>>>(*p);
-  else glue_fwd_kernel<float><<<grid, GL_NT, 0, st>>>(*p);
+  if (p->dtype == MLSTM_BF16) glue_fwd_kernel<__nv_bfloat16><<<grid, 32 * glue_warps(p->D), 0, st>>>(*p);
+  else glue_fwd_kernel<float><<<grid, 32 * glue_warps(p->D), 0, st>>>(*p);
   return done("glue_fwd");
 }
 
@@ -294,8 +302,8 @@ int mlstm_b200_glue_bwd(const mlstm_glue_params* p, void* cuda_stream) {
   cudaStream_t st = reinterpret_cast<cudaStream_t>(cuda_stream);
   const int grid = glue_grid(*p);
   float* ws = reinterpret_cast<float*>(p->workspace);
-  if (p->dtype == MLSTM_BF16) glue_bwd_kernel<__nv_bfloat16><<<grid, GL_NT, 0, st>>>(*p, ws);
-  else glue_bwd_kernel<float><<<grid, GL_NT, 0, st>>>(*p, ws);
+  if (p->dtype == MLSTM_BF16) glue_bwd_kernel<__nv_bfloat16><<<grid, 32 * glue_warps(p->D), 0, st>>>(*p, ws);
+  else glue_bwd_kernel<float><<<grid, 32 * glue_warps(p->D), 0, st>>>(*p, ws);
   if ((rc = done("glue_bwd"))) return rc;
   glue_reduce_kernel<<<(3 * p->D * 8 + 255) / 256, 256, 0, st>>>(*p, ws, grid);
   return done("glue_reduce");

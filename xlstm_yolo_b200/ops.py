@@ -414,6 +414,10 @@ def gate_proj_fwd_raw(q3, k3, v3, w_i, b_i, w_f, b_f, NH):
     f = torch.empty((B, S, NH), dtype=torch.float32, device=q3.device)
     g = _gate_params(q3, k3, v3, w_i, b_i, w_f, b_f, NH)
     g.i, g.f = i.data_ptr(), f.data_ptr()
+    need = lib.mlstm_b200_gates_fwd_workspace_bytes(C.byref(g))
+    if need:
+        ws = torch.empty((need + 15) // 16 * 4, dtype=torch.float32, device=q3.device)
+        g.workspace, g.workspace_bytes = ws.data_ptr(), ws.numel() * 4
     with torch.cuda.device(q3.device):
         rc = lib.mlstm_b200_gates_fwd(C.byref(g), _stream())
     if rc:
@@ -546,7 +550,7 @@ def glue_supported(h: torch.Tensor, c: torch.Tensor, z: torch.Tensor) -> bool:
         return False
     B, NH, S, DH = h.shape
     D = NH * DH
-    if not _glue_lib_ok(int(D), int(NH)):   # the C-side shape gate (D / 256 in {1, 2, 4, 8}, DH | 256)
+    if not _glue_lib_ok(int(D), int(NH)):   # the C-side shape gate (D % 256 == 0, D <= 2048, DH | 256)
         return False
     if h.stride() != (S * D, DH, D, 1) or not _aligned(h):
         return False
